@@ -210,17 +210,16 @@ def run_reference(args, wl, name):
     # One step = the workload's whole batch (the GPU arm's config: same_config), as
     # `passes` sweeps over a pool of distinct problems: 65 536 quadrotor problems would be
     # 11.6 GB of host arrays, the pool (<= 2 048 problems, 360 MB, far beyond the CPU caches) keeps
-    # the arm's set-up to seconds.  Steps are bounded to what a few minutes allow.
+    # the arm's set-up to seconds.  Warm-up is bounded to what half a minute allows.
     batch = wl["batch"]
     pool = min(batch, 2048)
     while batch % pool:
         pool -= 1
     passes = batch // pool
     host = host_problems(wl["n"], wl["m"], wl["T"], pool, seed=1234)
-    secs, _ = cpu_time_sample(wl, pool, cores, host=host)  # warm-up pass, sizes the run
+    secs, _ = cpu_time_sample(wl, pool, cores, host=host)  # warm-up pass, sizes the warm-up
     step_s = secs * passes
-    budget_s = 150.0
-    steps = max(1, min(args.steps, int(budget_s / max(step_s, 1e-9))))
+    steps = args.steps
     warm = max(0, min(args.warmup, int(30.0 / max(step_s, 1e-9))))
     for _ in range(warm):
         cpu_time_sample(wl, pool, cores, repeats=passes, host=host)
@@ -239,8 +238,8 @@ def run_reference(args, wl, name):
         "ms_per_step": 1e3 * total / steps, "higher_is_better": True, "scaling": args.scaling,
         "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": name, **wl, "batch": sample, "global_batch": sample,
-                   "note": "host CPU arm: the workload's whole batch per step; steps bounded to "
-                           "a few minutes of CPU time"},
+                   "note": "host CPU arm: the workload's whole batch per step; warm-up bounded "
+                           "to half a minute of CPU time"},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port",
                          "sample": desc},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -267,6 +266,44 @@ def load_traffic(name, kernels, batch):
         return None
 
 
+# --dump-outputs keeps the whole dump under DUMP_BYTES: when every problem does not fit, it writes
+# the rows np.sort(np.random.default_rng(DUMP_SEED).choice(batch, k, replace=False)) of every
+# per-problem array, so two builds run with the same arguments write the same problems.
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_SEED = 0
+
+
+def dump_outputs(directory, batch, per_problem, whole):
+    """Writes DIR/<name>.npy for the arrays the timed call returned in its last step.
+
+    per_problem: name -> device tensor, either [size, batch_stride] (engine layout, written as
+    [problems, size]) or [batch_stride] (one value per problem); whole: name -> device tensor
+    written as it is.  Floating arrays keep their precision, integer ones are written as float64.
+    """
+    import torch
+
+    def itemsize(t):
+        return t.element_size() if t.is_floating_point() else 8
+
+    fixed = sum(t.numel() * itemsize(t) for t in whole.values())
+    per_row = sum((t.shape[0] if t.dim() == 2 else 1) * itemsize(t) for t in per_problem.values())
+    headers = 256 * (len(per_problem) + len(whole))
+    k = min(batch, (DUMP_BYTES - headers - fixed) // per_row)
+    rows = np.arange(batch)
+    if k < batch:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(batch, k, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    arrays = dict(whole)
+    for name, t in per_problem.items():
+        idx = torch.from_numpy(rows).to(t.device)
+        arrays[name] = t[:, idx].T if t.dim() == 2 else t[idx]
+    for name, t in arrays.items():
+        t = t if t.is_floating_point() else t.to(torch.float64)
+        np.save(os.path.join(directory, f"{name}.npy"), t.contiguous().cpu().numpy())
+    print(f"bench: wrote {len(arrays)} arrays of the last timed step to {directory} "
+          f"({k} of {batch} problems)", file=sys.stderr)
+
+
 def run_ours(args, wl, name):
     import torch
     import torch.distributed as dist
@@ -279,6 +316,8 @@ def run_ours(args, wl, name):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the engine has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one process: run it with --gpus 1")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     if world > 1:
@@ -401,6 +440,13 @@ def run_ours(args, wl, name):
     ms_total = float(t.item())
     ms_per_step = ms_total / args.steps
     value = total_batch / (ms_per_step * 1e-3)
+
+    if args.dump_outputs:
+        sizes = eng.lqr_sizes
+        last = out32 if out32 is not None else out
+        dump_outputs(args.dump_outputs, batch,
+                     {**{k: last[k][:sizes[k]] for k in _capi.LQR_OUTPUT_FIELDS}, "status": status},
+                     {"stats": stats})
 
     # correctness outside the timed region: KKT residual of every problem
     if inp32 is not None:
@@ -682,6 +728,10 @@ def run_kkt(args):
                                       "ms_per_step": ms.value / args.steps}
     lib.sipoc_profile_enable(eng._handle, 0)
     sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, batch,
+                     {"sol": sol[:b_h.shape[1]], "ok": ok, "residual_norm": norms},
+                     {"stats": stats})
     st = stats.cpu().numpy()
     # relative residual: ||K sol - b|| / ||b|| (r2 up to 1e9 scales the rows)
     rel = (norms[:batch].cpu().numpy() / np.linalg.norm(b_h, axis=1)).max()
@@ -750,7 +800,15 @@ def main():
                     help="also time sipoc_lqr_factor_solve_host_packed (e2e.packed: Q / R as packed "
                          "lower triangles, M not sent)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the timed call returned in its "
+                         "last step as DIR/<name>.npy (float32 / float64, under 64 MB in all: a "
+                         "fixed sample of the problems when the batch is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload in ("newton_kkt", "newton_kkt_uniform"):
         return run_kkt(args)

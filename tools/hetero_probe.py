@@ -1,7 +1,8 @@
 """Timing of the reference's VariableLQRProblem benchmark shapes (lqr_benchmark.cpp:209-310: heterogeneous
 chain, star, binary tree) on the reference-order padded plans against the generic kernels."""
-import sys, time, numpy as np, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, time, numpy as np, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import problem_gen as pg
 from gpu_helpers import *
 from oracle import pyoracle

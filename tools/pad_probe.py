@@ -1,5 +1,6 @@
-import sys, numpy as np
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, numpy as np
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import problem_gen as pg
 from gpu_helpers import *
 from test_gpu_kkt import _gpu_kkt, rel_err
