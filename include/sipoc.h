@@ -246,6 +246,44 @@ sipoc_error sipoc_lqr_residual(sipoc_engine *engine, const sipoc_lqr_input *in,
 sipoc_error sipoc_status_stats(sipoc_engine *engine, const int *status, double *stats,
                                void *stream);
 
+/* ---- reverse-mode derivative of the LQR solve ------------------------------------------
+ * The solve is K z = -h with z = (x, u, y), h = (q, r, c) and K symmetric.  For a cotangent
+ * g = (g_x, g_u, g_y) = dL/d(x, u, y), sipoc_lqr_vjp writes the adjoint mu = -K^-1 g (the same
+ * LQR solved with (q, r, c) := g) and, from dL = mu' (dK z + dh), the gradient of L with
+ * respect to every input array, per problem, in that array's own layout:
+ *   q, r, c : mu_x, mu_u, mu_y          delta_i : -mu_y_i .* y_i  (every node, root included)
+ *   Q_i : (mu_x_i x_i' + x_i mu_x_i') / 2          R_e : (mu_u_e u_e' + u_e mu_u_e') / 2
+ *   M_e : mu_x_p u_e' + x_p mu_u_e'                A_e : y_c mu_x_p' + mu_y_c x_p'
+ *   B_e : y_c mu_u_e' + mu_y_c u_e'                (p / c: parent / child node of edge e)
+ * Q and R get the gradient of the solve as a function of the SYMMETRIC matrices (the same
+ * values in both triangles), although the kernels read only lower triangles: it is what a
+ * caller who forms Q = (P + P') / 2 receives as dL/dQ.
+ *   in      : Q, M, R, A, B, delta of the forward; q, r, c are not read and may be NULL.
+ *   sol     : the forward's x, u, y.
+ *   cot     : required, all three arrays.
+ *   adjoint : caller-owned, receives mu (unspecified where status != 0).
+ *   grad    : required; any of its arrays may be NULL, and is then neither computed nor
+ *             written (a caller who wants dq / dc alone pays no matrix writes).
+ *   status  : device int[batch_stride] receiving the adjoint factorization's per-problem
+ *             FactorStatus, or NULL (an engine-owned buffer is used).
+ * Every requested gradient array is written in full: zeros in problems whose status != 0
+ * and in the padding lanes batch <= b < batch_stride, so every entry has a defined value.
+ * All arrays in the engine layout, 16-byte aligned as for the other device entry points.
+ * FP64 only.  The factorization is recomputed (the call keeps no state from the forward) on
+ * the plan the forward uses, and it replaces the handle's kept LQR factorization the way
+ * sipoc_lqr_factor_solve does.  The call only enqueues work on `stream`, so it can be
+ * recorded in a graph under the rules above. */
+typedef struct sipoc_lqr_cotangent {
+  const double *x, *u, *y;
+} sipoc_lqr_cotangent;
+typedef struct sipoc_lqr_grad {
+  double *Q, *M, *R, *q, *r, *A, *B, *c, *delta;
+} sipoc_lqr_grad;
+sipoc_error sipoc_lqr_vjp(sipoc_engine *engine, const sipoc_lqr_input *in,
+                          const sipoc_lqr_output *sol, const sipoc_lqr_cotangent *cot,
+                          const sipoc_lqr_output *adjoint, const sipoc_lqr_grad *grad,
+                          int *status, void *stream);
+
 /* ---- layout conversion (device <-> device) ------------------------------ */
 /* src: problem-major [batch][size]; dst: engine layout [size][batch_stride]. */
 sipoc_error sipoc_pack(sipoc_engine *engine, const double *src, double *dst,

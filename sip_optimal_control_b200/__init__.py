@@ -13,4 +13,14 @@ from .kkt import CallbackProvider  # noqa: F401
 from .lqr import LQR, Dimensions, Engine, FactorStatus, SipocError, Topology  # noqa: F401
 
 __all__ = ["LQR", "CallbackProvider", "Dimensions", "Topology", "Engine", "FactorStatus",
-           "SipocError", "LIB_PATH", "declared_symbols"]
+           "SipocError", "LIB_PATH", "declared_symbols", "autograd"]
+
+
+def __getattr__(name):
+    # ``autograd`` (torch.autograd binding of the LQR solve) imports torch, which the rest of
+    # the package loads only when it first touches a device: import it on first use.
+    if name == "autograd":
+        import importlib
+
+        return importlib.import_module(".autograd", __name__)
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

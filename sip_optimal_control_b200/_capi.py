@@ -67,6 +67,14 @@ class LqrOutput(ctypes.Structure):
     _fields_ = [(k, c_void_p) for k in LQR_OUTPUT_FIELDS]
 
 
+class LqrCotangent(ctypes.Structure):
+    _fields_ = [(k, c_void_p) for k in LQR_OUTPUT_FIELDS]
+
+
+class LqrGrad(ctypes.Structure):
+    _fields_ = [(k, c_void_p) for k in LQR_INPUT_FIELDS]
+
+
 KKT_THETA_FIELDS = ("node_hxt", "node_jct", "node_jgt", "node_htt", "edge_hxt", "edge_hut",
                     "edge_dynt", "edge_jct", "edge_jgt", "edge_htt")
 
@@ -155,6 +163,8 @@ def _load() -> ctypes.CDLL:
     lib.sipoc_lqr_solve_pm.argtypes = [E, LI, LO, P]
     lib.sipoc_lqr_factor_solve_pm.argtypes = [E, LI, LO, P, P]
     lib.sipoc_lqr_residual.argtypes = [E, LI, LO, P, P, P, P]
+    lib.sipoc_lqr_vjp.argtypes = [E, LI, LO, ctypes.POINTER(LqrCotangent), LO,
+                                  ctypes.POINTER(LqrGrad), P, P]
     lib.sipoc_status_stats.argtypes = [E, P, P, P]
     lib.sipoc_pack.argtypes = [E, P, P, ctypes.c_int64, P]
     lib.sipoc_unpack.argtypes = [E, P, P, ctypes.c_int64, P]

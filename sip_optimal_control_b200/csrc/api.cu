@@ -14,6 +14,7 @@
 #include "generic_kernels.cuh"
 #include "kkt_fast.cuh"
 #include "kkt_theta.cuh"
+#include "lqr_vjp.cuh"
 #include "scan.cuh"
 #include "model_scatter.cuh"
 #include "riccati_f32.cuh"
@@ -102,6 +103,7 @@ struct sipoc_engine {
   float *f32_store = nullptr;
   double *f64t_store = nullptr;
   double *h_packed = nullptr;  // packed-symmetric host entry: Q / R triangles before expansion
+  int *vjp_status = nullptr;   // status of sipoc_lqr_vjp when the caller passes none (lazy)
 
   // Parallel-in-time factor + solve (scan.cu): long uniform chains, small batches.
   struct Scan {
@@ -1261,6 +1263,40 @@ sipoc_error sipoc_lqr_residual(sipoc_engine *e, const sipoc_lqr_input *in,
   e->launches += stats != nullptr ? 2 : 1;
   sipoc_error rc = check_launch(e, "lqr_residual");
   return rc != SIPOC_OK ? rc : reduce_stats(e, stats, stream);
+}
+
+sipoc_error sipoc_lqr_vjp(sipoc_engine *e, const sipoc_lqr_input *in,
+                          const sipoc_lqr_output *sol, const sipoc_lqr_cotangent *cot,
+                          const sipoc_lqr_output *adjoint, const sipoc_lqr_grad *grad,
+                          int *status, void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (null_in(in, true, false) || sol == nullptr || !sol->x || !sol->u || !sol->y ||
+      cot == nullptr || !cot->x || !cot->u || !cot->y || adjoint == nullptr || !adjoint->x ||
+      !adjoint->u || !adjoint->y || grad == nullptr)
+    return fail(e, SIPOC_INVALID_ARGUMENT, "NULL LQR input / solution / cotangent / adjoint / grad");
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  sipoc_error rc;
+  if (status == nullptr) {
+    if (e->vjp_status == nullptr &&
+        (rc = dev_alloc(e, reinterpret_cast<void **>(&e->vjp_status),
+                        static_cast<size_t>(e->ld) * sizeof(int))) != SIPOC_OK)
+      return rc;
+    status = e->vjp_status;
+  }
+  // K is symmetric: the adjoint is the same LQR with the cotangent as (q, r, c).
+  const LqrIn adj_in{in->Q, in->M, in->R, cot->x, cot->u, in->A, in->B, cot->y, in->delta};
+  const LqrOut adj{adjoint->x, adjoint->u, adjoint->y};
+  if ((rc = lqr_factor_solve_core(e, adj_in, adj, status, s)) != SIPOC_OK) return rc;
+  const LqrGrad g{grad->Q, grad->M, grad->R, grad->q, grad->r, grad->A, grad->B, grad->c,
+                  grad->delta};
+  if (!g.Q && !g.M && !g.R && !g.q && !g.r && !g.A && !g.B && !g.c && !g.delta) return SIPOC_OK;
+  {
+    ProfScope ps(&e->prof, "lqr_vjp_kernel", s);
+    launch_lqr_vjp(e->dt, LqrOut{sol->x, sol->u, sol->y}, adj, status, g, e->batch, e->ld, s);
+  }
+  e->launches += 1;
+  return check_launch(e, "lqr_vjp");
 }
 
 sipoc_error sipoc_status_stats(sipoc_engine *e, const int *status, double *stats,

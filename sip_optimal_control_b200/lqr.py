@@ -386,6 +386,38 @@ class LQR:
                                             status.data_ptr(), e.stream_ptr(stream)))
         return status
 
+    def vjp(self, inp: dict, out: dict, cot: dict, want=None, adjoint=None, status=None,
+            stream=None) -> dict:
+        """Reverse-mode derivative of ``factor_solve`` (sipoc_lqr_vjp; include/sipoc.h).
+
+        ``inp`` and ``out`` are the forward's inputs and solution, ``cot`` holds dL/dx, dL/du,
+        dL/dy (engine layout, keys x, u, y).  ``want`` is the set of input names to
+        differentiate (default: all nine); the others are neither computed nor written.
+        Returns a dict with one engine-layout gradient tensor per wanted name, ``adjoint``
+        (dict x, u, y) and ``status`` (the adjoint factorization's FactorStatus per problem).
+        Q and R get the symmetric gradient; failed problems and padding lanes get zeros."""
+        e = self.engine
+        want = set(_capi.LQR_INPUT_FIELDS if want is None else want)
+        unknown = want - set(_capi.LQR_INPUT_FIELDS)
+        if unknown:
+            raise ValueError(f"not an LQR input: {sorted(unknown)}")
+        adjoint = self.alloc_output() if adjoint is None else adjoint
+        status = e.empty_int() if status is None else status
+        grads = {k: e.empty(e.lqr_sizes[k]) for k in _capi.LQR_INPUT_FIELDS if k in want}
+        si, ss, sa = _lqr_input_struct(inp), _lqr_output_struct(out), _lqr_output_struct(adjoint)
+        sc = _capi.LqrCotangent()
+        for k in _capi.LQR_OUTPUT_FIELDS:
+            setattr(sc, k, cot[k].data_ptr())
+        sg = _capi.LqrGrad()
+        for k in _capi.LQR_INPUT_FIELDS:
+            setattr(sg, k, grads[k].data_ptr() if k in grads else None)
+        e._check(lib.sipoc_lqr_vjp(e._handle, ctypes.byref(si), ctypes.byref(ss),
+                                   ctypes.byref(sc), ctypes.byref(sa), ctypes.byref(sg),
+                                   status.data_ptr(), e.stream_ptr(stream)))
+        grads["adjoint"] = adjoint
+        grads["status"] = status
+        return grads
+
     # -- optional FP32 mode (sipoc_lqr_factor_solve_f32; include/sipoc.h) -------------------
     @property
     def f32_supported(self) -> bool:
