@@ -393,6 +393,65 @@ sipoc_error sipoc_kkt_residual(sipoc_engine *engine, const sipoc_kkt_model *mode
                                const double *r3, const double *sol, const double *b,
                                const int *ok, double *residual_norm, double *stats,
                                void *stream);
+
+/* ---- reverse-mode derivative of the Newton-KKT solve -----------------------------------
+ * sipoc_kkt_solve computes sol = K^-1 b with K(w, r1, r2, r3) the operator of
+ * sipoc_kkt_apply:
+ *   K = [ H + diag(r1)   C'           G'            ]
+ *       [ C              -diag(r2)    0             ]
+ *       [ G              0            -diag(w + r3) ]
+ * K is symmetric.  For a cotangent g = dL/dsol, sipoc_kkt_vjp writes the adjoint
+ * lam = K^-1 g (the same KKT solve with b := g) and, from dL = lam' db - lam' dK sol, the
+ * gradient of L with respect to every model block, b and the regularization vectors, per
+ * problem, in each array's own layout.  With s_R, lam_R the rows of sol, lam in a row range R
+ * of [x | y | z], a block at K[R, C] (its transpose at K[C, R]) gets
+ *   -(lam_R s_C' + s_R lam_C')            off-diagonal blocks
+ *   -(lam_R s_R' + s_R lam_R') / 2        the symmetric Hessian blocks (R == C)
+ * at (p / c: parent / child node of edge e; theta: the theta rows of x)
+ *   node_hxx_i  x_state(i) x x_state(i)  sym     edge_hxx_e  x_state(p) x x_state(p)  sym
+ *   edge_hxu_e  x_state(p) x x_control(e)        edge_huu_e  x_control(e) x x_control(e) sym
+ *   edge_A_e, edge_B_e    y_dyn(c) x x_state(p), x_control(e)
+ *   node_jc_i, node_jg_i  y_node_c(i), z_node(i) x x_state(i)
+ *   edge_jcx_e, edge_jcu_e  y_edge_c(e) x x_state(p), x_control(e)
+ *   edge_jgx_e, edge_jgu_e  z_edge(e) x x_state(p), x_control(e)
+ *   node_hxt, node_jct, node_jgt  x_state(i), y_node_c(i), z_node(i) x theta
+ *   edge_hxt, edge_hut, edge_dynt, edge_jct, edge_jgt
+ *                         x_state(p), x_control(e), y_dyn(c), y_edge_c(e), z_edge(e) x theta
+ *   node_htt_i, edge_htt_e  theta x theta  sym (every copy gets the same value)
+ * and the vectors  db = lam,  dr1 = -lam_x .* s_x (theta rows included),
+ * dr2 = lam_y .* s_y,  dw = dr3 = lam_z .* s_z.  The -I couplings of the dynamics rows are
+ * constants.  Symmetric blocks get the gradient with respect to the SYMMETRIC matrix (the
+ * same values in both triangles): what a caller who forms H = (P + P') / 2 receives as dL/dH.
+ *   model, w, r1, r2, r3 : those of the forward (validated as by sipoc_kkt_factor).
+ *   sol     : the forward's solution;  cot : dL/dsol, required.
+ *   adjoint : caller-owned [x | y | z] vector, required, receives lam (unspecified where
+ *             ok == 0).
+ *   grad    : required; any of its arrays may be NULL, and is then neither computed nor
+ *             written; theta may be NULL (no theta gradient).  w and r3 may be one array.
+ *   ok      : device int[batch_stride] receiving the factorization's per-problem flags (as
+ *             sipoc_kkt_factor), or NULL (an engine-owned buffer is used).
+ * Every requested gradient array is written in full: zeros in problems whose ok == 0 and in
+ * the padding lanes batch <= b < batch_stride.  All arrays in the engine layout.  FP64 only.
+ * The factorization is recomputed on (model, w, r1, r2, r3) -- the call keeps no state from
+ * the forward -- on the plan sipoc_kkt_factor uses, and it replaces the handle's kept KKT
+ * factorization the way sipoc_kkt_factor does.  The call only enqueues work on `stream`, so
+ * it can be recorded in a graph under the rules above. */
+typedef struct sipoc_kkt_theta_grad {
+  double *node_hxt, *node_jct, *node_jgt, *node_htt;
+  double *edge_hxt, *edge_hut, *edge_dynt, *edge_jct, *edge_jgt, *edge_htt;
+} sipoc_kkt_theta_grad;
+typedef struct sipoc_kkt_grad {
+  double *node_hxx, *node_jc, *node_jg;
+  double *edge_hxx, *edge_hxu, *edge_huu, *edge_A, *edge_B;
+  double *edge_jcx, *edge_jcu, *edge_jgx, *edge_jgu;
+  const sipoc_kkt_theta_grad *theta; /* NULL: no theta gradient */
+  double *b, *w, *r1, *r2, *r3;
+} sipoc_kkt_grad;
+sipoc_error sipoc_kkt_vjp(sipoc_engine *engine, const sipoc_kkt_model *model, const double *w,
+                          const double *r1, const double *r2, const double *r3,
+                          const double *sol, const double *cot, double *adjoint,
+                          const sipoc_kkt_grad *grad, int *ok, void *stream);
+
 /* ---- optional FP32 mode ----------------------------------------------------------------
  * north_star: "an optional FP32 mode is reported separately with its own stated tolerance".
  * Factor + solve (LQR::factor + LQR::solve, lqr.hpp:192-194) entirely in single precision:

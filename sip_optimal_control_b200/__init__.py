@@ -17,7 +17,7 @@ __all__ = ["LQR", "CallbackProvider", "Dimensions", "Topology", "Engine", "Facto
 
 
 def __getattr__(name):
-    # ``autograd`` (torch.autograd binding of the LQR solve) imports torch, which the rest of
+    # ``autograd`` (torch.autograd bindings of the LQR and KKT solves) imports torch, which the rest of
     # the package loads only when it first touches a device: import it on first use.
     if name == "autograd":
         import importlib

@@ -93,6 +93,20 @@ class KktModel(ctypes.Structure):
         [("theta", ctypes.POINTER(KktThetaModel))]
 
 
+KKT_VECTOR_GRAD_FIELDS = ("b", "w", "r1", "r2", "r3")
+# every array sipoc_kkt_vjp can differentiate (sipoc_kkt_grad and its theta part)
+KKT_GRAD_FIELDS = KKT_MODEL_FIELDS + KKT_THETA_FIELDS + KKT_VECTOR_GRAD_FIELDS
+
+
+class KktThetaGrad(ctypes.Structure):
+    _fields_ = [(k, c_void_p) for k in KKT_THETA_FIELDS]
+
+
+class KktGrad(ctypes.Structure):
+    _fields_ = [(k, c_void_p) for k in KKT_MODEL_FIELDS] + \
+        [("theta", ctypes.POINTER(KktThetaGrad))] + [(k, c_void_p) for k in KKT_VECTOR_GRAD_FIELDS]
+
+
 MODEL_VALUE_FIELDS = ("node_f", "node_df_dx", "node_df_dtheta", "node_c", "node_g", "edge_f",
                       "edge_df_dx", "edge_df_du", "edge_df_dtheta", "edge_dyn_res", "edge_c",
                       "edge_g")
@@ -178,6 +192,7 @@ def _load() -> ctypes.CDLL:
     lib.sipoc_kkt_solve.argtypes = [E, KM, P, P, P]
     lib.sipoc_kkt_apply.argtypes = [E, KM, P, P, P, P, P, P, P]
     lib.sipoc_kkt_apply_block.argtypes = [E, KM, ctypes.c_int, P, P, P]
+    lib.sipoc_kkt_vjp.argtypes = [E, KM, P, P, P, P, P, P, P, ctypes.POINTER(KktGrad), P, P]
     lib.sipoc_kkt_apply_block_host.argtypes = [E, ctypes.c_int, P, P]
     lib.sipoc_lqr_factor_solve_host_packed.argtypes = [E, LI, LO, P]
     lib.sipoc_f32_supported.argtypes = [E]

@@ -6,6 +6,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
+#include <iterator>
 #include <new>
 #include <string>
 #include <vector>
@@ -14,6 +15,7 @@
 #include "generic_kernels.cuh"
 #include "kkt_fast.cuh"
 #include "kkt_theta.cuh"
+#include "kkt_vjp.cuh"
 #include "lqr_vjp.cuh"
 #include "scan.cuh"
 #include "model_scatter.cuh"
@@ -103,7 +105,7 @@ struct sipoc_engine {
   float *f32_store = nullptr;
   double *f64t_store = nullptr;
   double *h_packed = nullptr;  // packed-symmetric host entry: Q / R triangles before expansion
-  int *vjp_status = nullptr;   // status of sipoc_lqr_vjp when the caller passes none (lazy)
+  int *vjp_status = nullptr;   // status / ok of sipoc_*_vjp when the caller passes none (lazy)
 
   // Parallel-in-time factor + solve (scan.cu): long uniform chains, small batches.
   struct Scan {
@@ -1265,6 +1267,18 @@ sipoc_error sipoc_lqr_residual(sipoc_engine *e, const sipoc_lqr_input *in,
   return rc != SIPOC_OK ? rc : reduce_stats(e, stats, stream);
 }
 
+// The per-problem flags of a VJP call whose caller passes none: an engine-owned buffer.
+static sipoc_error default_vjp_status(sipoc_engine *e, int **status) {
+  if (*status != nullptr) return SIPOC_OK;
+  if (e->vjp_status == nullptr) {
+    const sipoc_error rc = dev_alloc(e, reinterpret_cast<void **>(&e->vjp_status),
+                                     static_cast<size_t>(e->ld) * sizeof(int));
+    if (rc != SIPOC_OK) return rc;
+  }
+  *status = e->vjp_status;
+  return SIPOC_OK;
+}
+
 sipoc_error sipoc_lqr_vjp(sipoc_engine *e, const sipoc_lqr_input *in,
                           const sipoc_lqr_output *sol, const sipoc_lqr_cotangent *cot,
                           const sipoc_lqr_output *adjoint, const sipoc_lqr_grad *grad,
@@ -1277,13 +1291,7 @@ sipoc_error sipoc_lqr_vjp(sipoc_engine *e, const sipoc_lqr_input *in,
   DeviceGuard guard(e->device);
   const cudaStream_t s = static_cast<cudaStream_t>(stream);
   sipoc_error rc;
-  if (status == nullptr) {
-    if (e->vjp_status == nullptr &&
-        (rc = dev_alloc(e, reinterpret_cast<void **>(&e->vjp_status),
-                        static_cast<size_t>(e->ld) * sizeof(int))) != SIPOC_OK)
-      return rc;
-    status = e->vjp_status;
-  }
+  if ((rc = default_vjp_status(e, &status)) != SIPOC_OK) return rc;
   // K is symmetric: the adjoint is the same LQR with the cotangent as (q, r, c).
   const LqrIn adj_in{in->Q, in->M, in->R, cot->x, cot->u, in->A, in->B, cot->y, in->delta};
   const LqrOut adj{adjoint->x, adjoint->u, adjoint->y};
@@ -1511,6 +1519,45 @@ sipoc_error sipoc_kkt_apply(sipoc_engine *e, const sipoc_kkt_model *model, const
   DeviceGuard guard(e->device);
   return kkt_apply_core(e, to_model(model), to_theta(model), w, r1, r2, r3, x, y,
                         static_cast<cudaStream_t>(stream));
+}
+
+sipoc_error sipoc_kkt_vjp(sipoc_engine *e, const sipoc_kkt_model *model, const double *w,
+                          const double *r1, const double *r2, const double *r3,
+                          const double *sol, const double *cot, double *adjoint,
+                          const sipoc_kkt_grad *grad, int *ok, void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (model_has_null(model) || theta_has_null(e, model) || !w || !r1 || !r2 || !r3 || !sol ||
+      !cot || !adjoint || grad == nullptr)
+    return fail(e, SIPOC_INVALID_ARGUMENT, "NULL KKT VJP argument");
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  sipoc_error rc;
+  if ((rc = default_vjp_status(e, &ok)) != SIPOC_OK) return rc;
+  // K is symmetric: the adjoint is the same KKT solve with b := cot.
+  const KktModel mdl = to_model(model);
+  if ((rc = kkt_factor_core(e, mdl, to_theta(model), w, r1, r2, r3, ok, s)) != SIPOC_OK) return rc;
+  if ((rc = kkt_solve_core(e, mdl, cot, adjoint, s)) != SIPOC_OK) return rc;
+  const sipoc_kkt_theta_grad no_theta{};
+  const sipoc_kkt_theta_grad &tg = grad->theta != nullptr ? *grad->theta : no_theta;
+  const KktGrad g{grad->node_hxx, grad->node_jc,  grad->node_jg,  grad->edge_hxx, grad->edge_hxu,
+                  grad->edge_huu, grad->edge_A,   grad->edge_B,   grad->edge_jcx, grad->edge_jcu,
+                  grad->edge_jgx, grad->edge_jgu, tg.node_hxt,    tg.node_jct,    tg.node_jgt,
+                  tg.node_htt,    tg.edge_hxt,    tg.edge_hut,    tg.edge_dynt,   tg.edge_jct,
+                  tg.edge_jgt,    tg.edge_htt,    grad->b,        grad->w,        grad->r1,
+                  grad->r2,       grad->r3};
+  const double *const arrays[] = {
+      g.node_hxx, g.node_jc,  g.node_jg,  g.edge_hxx,  g.edge_hxu, g.edge_huu, g.edge_A,
+      g.edge_B,   g.edge_jcx, g.edge_jcu, g.edge_jgx,  g.edge_jgu, g.node_hxt, g.node_jct,
+      g.node_jgt, g.node_htt, g.edge_hxt, g.edge_hut,  g.edge_dynt, g.edge_jct, g.edge_jgt,
+      g.edge_htt, g.b,        g.w,        g.r1,        g.r2,       g.r3};
+  if (std::all_of(std::begin(arrays), std::end(arrays), [](const double *a) { return !a; }))
+    return SIPOC_OK;
+  {
+    ProfScope ps(&e->prof, "kkt_vjp_kernel", s);
+    launch_kkt_vjp(e->dt, sol, adjoint, ok, g, e->batch, e->ld, s);
+  }
+  e->launches += 1;
+  return check_launch(e, "kkt_vjp");
 }
 
 namespace {

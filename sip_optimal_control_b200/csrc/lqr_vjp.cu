@@ -4,57 +4,24 @@
 // store of a warp is 32 consecutive doubles; each block row of the grid (blockIdx.y) owns
 // one node (Q, q, c, delta) or one edge (M, R, r, A, B).  The entries of x, u, y and mu a
 // block needs are a few percent of what it writes: they are read through L1 and the rows
-// of an outer product are held in registers, kRows at a time, so the kernel is bound by
-// its gradient stores.
+// of an outer product are held in registers (vjp_common.cuh), so the kernel is bound by its
+// gradient stores.
 #include "lqr_vjp.cuh"
 
 #include <algorithm>
+
+#include "vjp_common.cuh"
 
 namespace sipoc {
 
 namespace {
 
 constexpr int kThreads = 128;
-constexpr int kRows = 8;         // rows of an outer-product block held in registers
 constexpr int kMaxGridY = 65535;
 
-// One problem's lane of an engine-layout vector; reads 0 where the problem is not live
-// (padding lane or failed factorization), so every gradient there comes out as zero.
-struct Lane {
-  const double *p;
-  size_t ld;
-  bool live;
-  __device__ __forceinline__ double operator()(int off) const {
-    return live ? __ldg(p + static_cast<size_t>(off) * ld) : 0.0;
-  }
-};
-
-__device__ __forceinline__ void copy_vec(double *G, size_t ld, int off, int n, const Lane &v) {
-  for (int i = 0; i < n; ++i) G[static_cast<size_t>(off + i) * ld] = v(off + i);
-}
-
-// G[off + i + j rows] = s (a_i b_j + c_i d_j): a rows x cols column-major block; a, c are
-// read at ra + i, b, d at cb + j.
-__device__ __forceinline__ void outer2(double *G, size_t ld, int off, int rows, int cols,
-                                       int ra, const Lane &a, const Lane &c, int cb,
-                                       const Lane &b, const Lane &d, double s) {
-  for (int i0 = 0; i0 < rows; i0 += kRows) {
-    double av[kRows], cv[kRows];
-#pragma unroll
-    for (int k = 0; k < kRows; ++k) {
-      const bool in = i0 + k < rows;
-      av[k] = in ? a(ra + i0 + k) : 0.0;
-      cv[k] = in ? c(ra + i0 + k) : 0.0;
-    }
-    for (int j = 0; j < cols; ++j) {
-      const double bj = b(cb + j), dj = d(cb + j);
-      double *col = G + static_cast<size_t>(off + i0 + j * rows) * ld;
-#pragma unroll
-      for (int k = 0; k < kRows; ++k)
-        if (i0 + k < rows) col[k * ld] = s * (av[k] * bj + cv[k] * dj);
-    }
-  }
-}
+using vjp::Lane;
+using vjp::copy_vec;
+using vjp::outer2;
 
 __global__ void __launch_bounds__(kThreads)
 lqr_vjp_kernel(DevTables t, LqrOut sol, LqrOut adj, const int *status, LqrGrad g,

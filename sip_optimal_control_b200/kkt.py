@@ -182,6 +182,53 @@ class CallbackProvider:
             e.stream_ptr(stream)))
         return norms, stats
 
+    def vjp(self, model: dict, w, r1, r2, r3, sol, cot, want=None, ok=None, stream=None) -> dict:
+        """Reverse-mode derivative of ``factor`` + ``solve`` (sipoc_kkt_vjp; include/sipoc.h).
+
+        ``model``, ``w``, ``r1``, ``r2``, ``r3`` are the forward's inputs and ``sol`` its
+        solution, ``cot`` is dL/dsol (engine layout).  ``want`` is the set of names to
+        differentiate among ``_capi.KKT_GRAD_FIELDS`` (default: all of them, the theta blocks
+        when theta_dim > 0); the others are neither computed nor written.  Returns a dict with
+        one engine-layout gradient tensor per wanted name, ``adjoint`` (lam = K^-1 cot) and
+        ``ok`` (the factorization's per-problem flags).  Symmetric Hessian blocks get the
+        symmetric gradient; problems with ok == 0 and padding lanes get zeros."""
+        e = self.engine
+        if not self.input_is_valid_:
+            raise SipocError(self.engine.create_status, "vjp on an invalid structure")
+        sizes = self.sizes
+        theta = sizes["theta_dim"] > 0
+        fields = _capi.KKT_MODEL_FIELDS + (_capi.KKT_THETA_FIELDS if theta else ()) + \
+            _capi.KKT_VECTOR_GRAD_FIELDS
+        want = set(fields if want is None else want)
+        unknown = want - set(fields)
+        if unknown:
+            raise ValueError(f"not a differentiable KKT input: {sorted(unknown)}")
+        vec_size = dict(b=sizes["kkt_dim"], w=sizes["z_dim"], r1=sizes["x_dim"],
+                        r2=sizes["y_dim"], r3=sizes["z_dim"])
+        size = {k: vec_size.get(k, sizes.get(k, 0)) for k in fields}
+        # an empty array is one row of zeros, as Engine.pack makes it
+        grads = {k: e.empty(size[k]) if size[k] else e.zeros(0) for k in fields if k in want}
+        adjoint = e.empty(sizes["kkt_dim"])
+        ok = e.empty_int() if ok is None else ok
+        keep = []
+        m = _model_struct(model, False, keep)
+        sg = _capi.KktGrad()
+        for k in _capi.KKT_MODEL_FIELDS + _capi.KKT_VECTOR_GRAD_FIELDS:
+            setattr(sg, k, grads[k].data_ptr() if k in grads else None)
+        if theta and want & set(_capi.KKT_THETA_FIELDS):
+            st = _capi.KktThetaGrad()
+            for k in _capi.KKT_THETA_FIELDS:
+                setattr(st, k, grads[k].data_ptr() if k in grads else None)
+            keep.append(st)
+            sg.theta = ctypes.pointer(st)
+        e._check(lib.sipoc_kkt_vjp(e._handle, ctypes.byref(m), w.data_ptr(), r1.data_ptr(),
+                                   r2.data_ptr(), r3.data_ptr(), sol.data_ptr(), cot.data_ptr(),
+                                   adjoint.data_ptr(), ctypes.byref(sg), ok.data_ptr(),
+                                   e.stream_ptr(stream)))
+        grads["adjoint"] = adjoint
+        grads["ok"] = ok
+        return grads
+
     def capture_step(self, model: dict, w, r1, r2, r3, b, sol, ok=None) -> "CapturedKktStep":
         """factor + solve + residual (one Newton-KKT iteration's linear algebra,
         sip_optimal_control.cpp:129-145) recorded once as a CUDA graph over the given device
