@@ -9,7 +9,7 @@ CSRC := sip_optimal_control_b200/csrc
 LIBDIR := sip_optimal_control_b200/lib
 OBJDIR := build/obj
 SRCS := $(CSRC)/api.cu $(CSRC)/generic_kernels.cu $(CSRC)/riccati_fast.cu $(CSRC)/riccati_cta.cu $(CSRC)/riccati_strict.cu $(CSRC)/kkt_fast.cu $(CSRC)/kkt_theta.cu $(CSRC)/comm.cu $(CSRC)/scan.cu $(CSRC)/model_scatter.cu $(CSRC)/riccati_f32.cu \
-        $(CSRC)/lqr_vjp.cu $(CSRC)/kkt_vjp.cu $(CSRC)/workload.cu $(CSRC)/structure.cpp
+        $(CSRC)/lqr_vjp.cu $(CSRC)/kkt_vjp.cu $(CSRC)/jvp.cu $(CSRC)/workload.cu $(CSRC)/structure.cpp
 OBJS := $(patsubst $(CSRC)/%,$(OBJDIR)/%.o,$(SRCS)) $(OBJDIR)/riccati_fast_part1.cu.o \
         $(OBJDIR)/riccati_fast_part2.cu.o $(OBJDIR)/riccati_fast_part3.cu.o
 HDRS := $(wildcard $(CSRC)/*.cuh $(CSRC)/*.hpp) include/sipoc.h

@@ -284,6 +284,30 @@ sipoc_error sipoc_lqr_vjp(sipoc_engine *engine, const sipoc_lqr_input *in,
                           const sipoc_lqr_output *adjoint, const sipoc_lqr_grad *grad,
                           int *status, void *stream);
 
+/* ---- forward-mode derivative of the LQR solve ------------------------------------------
+ * From K z = -h, tangents (dK, dh) of the inputs move the solution by dz = -K^-1 (dK z + dh):
+ * the same LQR solved with (q, r, c) := t = dK z + dh.  sipoc_lqr_jvp builds t per problem
+ *   t_x_i = dQ_i x_i + dq_i + sum over the edges e with parent(e) = i of (dM_e u_e + dA_e' y_c)
+ *   t_u_e = dR_e u_e + dr_e + dM_e' x_p + dB_e' y_c
+ *   t_y_c = dA_e x_p + dB_e u_e - ddelta_c .* y_c + dc_c      (root: -ddelta_r .* y_r + dc_r)
+ * (p / c: parent / child node of edge e) and solves for dz = (dx, du, dy).  dQ and dR enter
+ * through their symmetric parts (dQ + dQ') / 2, read as full matrices: the exact transpose of
+ * the symmetric gradient of sipoc_lqr_vjp, so <JVP(t), g> = <t, VJP(g)> for every tangent.
+ *   in      : Q, M, R, A, B, delta of the forward; q, r, c are not read and may be NULL.
+ *   sol     : the forward's x, u, y.
+ *   tangent : required; any of its nine arrays may be NULL (a zero tangent: not read).
+ *   rhs     : caller-owned (q, r, c)-shaped arrays, required, receiving t (zeros in the
+ *             padding lanes batch <= b < batch_stride).
+ *   dsol    : caller-owned, required, receives (dx, du, dy).
+ *   status  : as for sipoc_lqr_vjp (the factorization's per-problem FactorStatus, or NULL).
+ * dsol is written in full: zeros in problems whose status != 0 and in the padding lanes.
+ * Everything else as for sipoc_lqr_vjp: engine layout, FP64, the factorization recomputed on
+ * the forward's plan (replacing the handle's kept one), graph-capturable. */
+sipoc_error sipoc_lqr_jvp(sipoc_engine *engine, const sipoc_lqr_input *in,
+                          const sipoc_lqr_output *sol, const sipoc_lqr_input *tangent,
+                          const sipoc_lqr_output *rhs, const sipoc_lqr_output *dsol,
+                          int *status, void *stream);
+
 /* ---- layout conversion (device <-> device) ------------------------------ */
 /* src: problem-major [batch][size]; dst: engine layout [size][batch_stride]. */
 sipoc_error sipoc_pack(sipoc_engine *engine, const double *src, double *dst,
@@ -451,6 +475,34 @@ sipoc_error sipoc_kkt_vjp(sipoc_engine *engine, const sipoc_kkt_model *model, co
                           const double *r1, const double *r2, const double *r3,
                           const double *sol, const double *cot, double *adjoint,
                           const sipoc_kkt_grad *grad, int *ok, void *stream);
+
+/* ---- forward-mode derivative of the Newton-KKT solve -----------------------------------
+ * From sol = K^-1 b, tangents of the inputs move the solution by d sol = K^-1 (db - dK sol):
+ * the same KKT solve with b := t = db - dK sol.  dK holds the tangent model blocks where the
+ * table of sipoc_kkt_vjp places them (every copy of node_htt / edge_htt adds to the theta x
+ * theta block), diag(dr1) on the x rows (theta rows included), -diag(dr2) on the y rows and
+ * -diag(dw + dr3) on the z rows; the -I couplings of the dynamics rows are constants.  The
+ * symmetric Hessian blocks enter through their symmetric parts (dB + dB') / 2, read as full
+ * matrices: the exact transpose of the symmetric gradient of sipoc_kkt_vjp.
+ *   model, w, r1, r2, r3 : those of the forward (validated as by sipoc_kkt_factor).
+ *   sol     : the forward's solution.
+ *   tangent : required; every block pointer, model.theta, and b, w, r1, r2, r3 may be NULL
+ *             (a zero tangent: not read).  w and r3 may be one array, here and in the forward.
+ *   rhs     : caller-owned [x | y | z] vector, required, receiving t (zeros in the padding
+ *             lanes).
+ *   dsol    : caller-owned [x | y | z] vector, required, receives d sol.
+ *   ok      : as for sipoc_kkt_vjp.
+ * dsol is written in full: zeros in problems whose ok == 0 and in the padding lanes.
+ * Everything else as for sipoc_kkt_vjp: engine layout, FP64, the factorization recomputed on
+ * the forward's plan (replacing the handle's kept one), graph-capturable. */
+typedef struct sipoc_kkt_tangent {
+  sipoc_kkt_model model;
+  const double *b, *w, *r1, *r2, *r3;
+} sipoc_kkt_tangent;
+sipoc_error sipoc_kkt_jvp(sipoc_engine *engine, const sipoc_kkt_model *model, const double *w,
+                          const double *r1, const double *r2, const double *r3,
+                          const double *sol, const sipoc_kkt_tangent *tangent, double *rhs,
+                          double *dsol, int *ok, void *stream);
 
 /* ---- optional FP32 mode ----------------------------------------------------------------
  * north_star: "an optional FP32 mode is reported separately with its own stated tolerance".

@@ -107,6 +107,11 @@ class KktGrad(ctypes.Structure):
         [("theta", ctypes.POINTER(KktThetaGrad))] + [(k, c_void_p) for k in KKT_VECTOR_GRAD_FIELDS]
 
 
+# sipoc_kkt_tangent: a tangent of every array of KKT_GRAD_FIELDS
+class KktTangent(ctypes.Structure):
+    _fields_ = [("model", KktModel)] + [(k, c_void_p) for k in KKT_VECTOR_GRAD_FIELDS]
+
+
 MODEL_VALUE_FIELDS = ("node_f", "node_df_dx", "node_df_dtheta", "node_c", "node_g", "edge_f",
                       "edge_df_dx", "edge_df_du", "edge_df_dtheta", "edge_dyn_res", "edge_c",
                       "edge_g")
@@ -179,6 +184,7 @@ def _load() -> ctypes.CDLL:
     lib.sipoc_lqr_residual.argtypes = [E, LI, LO, P, P, P, P]
     lib.sipoc_lqr_vjp.argtypes = [E, LI, LO, ctypes.POINTER(LqrCotangent), LO,
                                   ctypes.POINTER(LqrGrad), P, P]
+    lib.sipoc_lqr_jvp.argtypes = [E, LI, LO, LI, LO, LO, P, P]
     lib.sipoc_status_stats.argtypes = [E, P, P, P]
     lib.sipoc_pack.argtypes = [E, P, P, ctypes.c_int64, P]
     lib.sipoc_unpack.argtypes = [E, P, P, ctypes.c_int64, P]
@@ -193,6 +199,7 @@ def _load() -> ctypes.CDLL:
     lib.sipoc_kkt_apply.argtypes = [E, KM, P, P, P, P, P, P, P]
     lib.sipoc_kkt_apply_block.argtypes = [E, KM, ctypes.c_int, P, P, P]
     lib.sipoc_kkt_vjp.argtypes = [E, KM, P, P, P, P, P, P, P, ctypes.POINTER(KktGrad), P, P]
+    lib.sipoc_kkt_jvp.argtypes = [E, KM, P, P, P, P, P, ctypes.POINTER(KktTangent), P, P, P, P]
     lib.sipoc_kkt_apply_block_host.argtypes = [E, ctypes.c_int, P, P]
     lib.sipoc_lqr_factor_solve_host_packed.argtypes = [E, LI, LO, P]
     lib.sipoc_f32_supported.argtypes = [E]

@@ -15,6 +15,7 @@
 #include "generic_kernels.cuh"
 #include "kkt_fast.cuh"
 #include "kkt_theta.cuh"
+#include "jvp.cuh"
 #include "kkt_vjp.cuh"
 #include "lqr_vjp.cuh"
 #include "scan.cuh"
@@ -105,7 +106,7 @@ struct sipoc_engine {
   float *f32_store = nullptr;
   double *f64t_store = nullptr;
   double *h_packed = nullptr;  // packed-symmetric host entry: Q / R triangles before expansion
-  int *vjp_status = nullptr;   // status / ok of sipoc_*_vjp when the caller passes none (lazy)
+  int *vjp_status = nullptr;   // status / ok of sipoc_*_vjp / _jvp when the caller passes none (lazy)
 
   // Parallel-in-time factor + solve (scan.cu): long uniform chains, small batches.
   struct Scan {
@@ -1267,7 +1268,7 @@ sipoc_error sipoc_lqr_residual(sipoc_engine *e, const sipoc_lqr_input *in,
   return rc != SIPOC_OK ? rc : reduce_stats(e, stats, stream);
 }
 
-// The per-problem flags of a VJP call whose caller passes none: an engine-owned buffer.
+// The per-problem flags of a VJP / JVP call whose caller passes none: an engine-owned buffer.
 static sipoc_error default_vjp_status(sipoc_engine *e, int **status) {
   if (*status != nullptr) return SIPOC_OK;
   if (e->vjp_status == nullptr) {
@@ -1305,6 +1306,43 @@ sipoc_error sipoc_lqr_vjp(sipoc_engine *e, const sipoc_lqr_input *in,
   }
   e->launches += 1;
   return check_launch(e, "lqr_vjp");
+}
+
+sipoc_error sipoc_lqr_jvp(sipoc_engine *e, const sipoc_lqr_input *in,
+                          const sipoc_lqr_output *sol, const sipoc_lqr_input *tangent,
+                          const sipoc_lqr_output *rhs, const sipoc_lqr_output *dsol,
+                          int *status, void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (null_in(in, true, false) || sol == nullptr || !sol->x || !sol->u || !sol->y ||
+      tangent == nullptr || rhs == nullptr || !rhs->x || !rhs->u || !rhs->y || dsol == nullptr ||
+      !dsol->x || !dsol->u || !dsol->y)
+    return fail(e, SIPOC_INVALID_ARGUMENT, "NULL LQR input / solution / tangent / rhs / dsol");
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  sipoc_error rc;
+  if ((rc = default_vjp_status(e, &status)) != SIPOC_OK) return rc;
+  const LqrOut t{rhs->x, rhs->u, rhs->y}, d{dsol->x, dsol->u, dsol->y};
+  {
+    ProfScope ps(&e->prof, "lqr_jvp_kernel", s);
+    launch_lqr_jvp(e->dt, LqrOut{sol->x, sol->u, sol->y},
+                   LqrTangent{tangent->Q, tangent->M, tangent->R, tangent->q, tangent->r,
+                              tangent->A, tangent->B, tangent->c, tangent->delta},
+                   t, e->batch, e->ld, s);
+  }
+  e->launches += 1;
+  if ((rc = check_launch(e, "lqr_jvp")) != SIPOC_OK) return rc;
+  // The tangent is the same LQR with t as (q, r, c).
+  const LqrIn tan_in{in->Q, in->M, in->R, t.x, t.u, in->A, in->B, t.y, in->delta};
+  if ((rc = lqr_factor_solve_core(e, tan_in, d, status, s)) != SIPOC_OK) return rc;
+  {
+    ProfScope ps(&e->prof, "jvp_zero_dead_lanes", s);
+    const HostStructure &h = e->hs;
+    launch_zero_dead_lanes(d.x, h.n_off[h.N], status, false, e->batch, e->ld, s);
+    launch_zero_dead_lanes(d.u, h.m_off[h.E], status, false, e->batch, e->ld, s);
+    launch_zero_dead_lanes(d.y, h.n_off[h.N], status, false, e->batch, e->ld, s);
+  }
+  e->launches += 3;
+  return check_launch(e, "lqr_jvp zero pass");
 }
 
 sipoc_error sipoc_status_stats(sipoc_engine *e, const int *status, double *stats,
@@ -1558,6 +1596,43 @@ sipoc_error sipoc_kkt_vjp(sipoc_engine *e, const sipoc_kkt_model *model, const d
   }
   e->launches += 1;
   return check_launch(e, "kkt_vjp");
+}
+
+sipoc_error sipoc_kkt_jvp(sipoc_engine *e, const sipoc_kkt_model *model, const double *w,
+                          const double *r1, const double *r2, const double *r3,
+                          const double *sol, const sipoc_kkt_tangent *tangent, double *rhs,
+                          double *dsol, int *ok, void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (model_has_null(model) || theta_has_null(e, model) || !w || !r1 || !r2 || !r3 || !sol ||
+      tangent == nullptr || !rhs || !dsol)
+    return fail(e, SIPOC_INVALID_ARGUMENT, "NULL KKT JVP argument");
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  sipoc_error rc;
+  if ((rc = default_vjp_status(e, &ok)) != SIPOC_OK) return rc;
+  const sipoc_kkt_model &tm = tangent->model;
+  const KktThetaModel tt = to_theta(&tm);
+  const KktTangent d{tm.node_hxx, tm.node_jc,  tm.node_jg,  tm.edge_hxx,  tm.edge_hxu, tm.edge_huu,
+                     tm.edge_A,   tm.edge_B,   tm.edge_jcx, tm.edge_jcu,  tm.edge_jgx, tm.edge_jgu,
+                     tt.node_hxt, tt.node_jct, tt.node_jgt, tt.node_htt,  tt.edge_hxt, tt.edge_hut,
+                     tt.edge_dynt, tt.edge_jct, tt.edge_jgt, tt.edge_htt, tangent->b,  tangent->w,
+                     tangent->r1, tangent->r2, tangent->r3};
+  {
+    ProfScope ps(&e->prof, "kkt_jvp_kernel", s);
+    launch_kkt_jvp(e->dt, sol, d, rhs, e->batch, e->ld, s);
+  }
+  e->launches += 1;
+  if ((rc = check_launch(e, "kkt_jvp")) != SIPOC_OK) return rc;
+  // The tangent is the same KKT solve with b := t.
+  const KktModel mdl = to_model(model);
+  if ((rc = kkt_factor_core(e, mdl, to_theta(model), w, r1, r2, r3, ok, s)) != SIPOC_OK) return rc;
+  if ((rc = kkt_solve_core(e, mdl, rhs, dsol, s)) != SIPOC_OK) return rc;
+  {
+    ProfScope ps(&e->prof, "jvp_zero_dead_lanes", s);
+    launch_zero_dead_lanes(dsol, e->hs.kkt_dim, ok, true, e->batch, e->ld, s);
+  }
+  e->launches += 1;
+  return check_launch(e, "kkt_jvp zero pass");
 }
 
 namespace {

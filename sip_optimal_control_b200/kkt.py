@@ -229,6 +229,49 @@ class CallbackProvider:
         grads["ok"] = ok
         return grads
 
+    def jvp(self, model: dict, w, r1, r2, r3, sol, tan: dict, dsol=None, rhs=None, ok=None,
+            stream=None) -> dict:
+        """Forward-mode derivative of ``factor`` + ``solve`` (sipoc_kkt_jvp; include/sipoc.h).
+
+        ``model``, ``w``, ``r1``, ``r2``, ``r3`` are the forward's inputs and ``sol`` its
+        solution; ``tan`` holds the tangents of any subset of ``_capi.KKT_GRAD_FIELDS`` (the
+        theta blocks when theta_dim > 0; engine layout).  An absent name is a zero tangent and
+        is not read.  Returns a dict with ``sol`` (the tangent of the solution), ``rhs`` (the
+        right-hand side t = db - dK sol the tangent solve used) and ``ok``.  Symmetric Hessian
+        blocks enter through their symmetric parts; problems with ok == 0 and padding lanes
+        get a zero tangent."""
+        e = self.engine
+        if not self.input_is_valid_:
+            raise SipocError(self.engine.create_status, "jvp on an invalid structure")
+        sizes = self.sizes
+        theta = sizes["theta_dim"] > 0
+        fields = _capi.KKT_MODEL_FIELDS + (_capi.KKT_THETA_FIELDS if theta else ()) + \
+            _capi.KKT_VECTOR_GRAD_FIELDS
+        unknown = set(tan) - set(fields)
+        if unknown:
+            raise ValueError(f"not a differentiable KKT input: {sorted(unknown)}")
+        dsol = e.empty(sizes["kkt_dim"]) if dsol is None else dsol
+        rhs = e.empty(sizes["kkt_dim"]) if rhs is None else rhs
+        ok = e.empty_int() if ok is None else ok
+        keep = []
+        m = _model_struct(model, False, keep)
+        st = _capi.KktTangent()
+        for k in _capi.KKT_MODEL_FIELDS:
+            setattr(st.model, k, tan[k].data_ptr() if k in tan else None)
+        for k in _capi.KKT_VECTOR_GRAD_FIELDS:
+            setattr(st, k, tan[k].data_ptr() if k in tan else None)
+        if theta and set(tan) & set(_capi.KKT_THETA_FIELDS):
+            tt = _capi.KktThetaModel()
+            for k in _capi.KKT_THETA_FIELDS:
+                setattr(tt, k, tan[k].data_ptr() if k in tan else None)
+            keep.append(tt)
+            st.model.theta = ctypes.pointer(tt)
+        e._check(lib.sipoc_kkt_jvp(e._handle, ctypes.byref(m), w.data_ptr(), r1.data_ptr(),
+                                   r2.data_ptr(), r3.data_ptr(), sol.data_ptr(),
+                                   ctypes.byref(st), rhs.data_ptr(), dsol.data_ptr(),
+                                   ok.data_ptr(), e.stream_ptr(stream)))
+        return dict(sol=dsol, rhs=rhs, ok=ok)
+
     def capture_step(self, model: dict, w, r1, r2, r3, b, sol, ok=None) -> "CapturedKktStep":
         """factor + solve + residual (one Newton-KKT iteration's linear algebra,
         sip_optimal_control.cpp:129-145) recorded once as a CUDA graph over the given device

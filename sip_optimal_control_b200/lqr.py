@@ -418,6 +418,32 @@ class LQR:
         grads["status"] = status
         return grads
 
+    def jvp(self, inp: dict, out: dict, tan: dict, dsol=None, rhs=None, status=None,
+            stream=None) -> dict:
+        """Forward-mode derivative of ``factor_solve`` (sipoc_lqr_jvp; include/sipoc.h).
+
+        ``inp`` and ``out`` are the forward's inputs and solution, ``tan`` holds the tangents
+        of any subset of the nine input names (engine layout); an absent name is a zero
+        tangent and is not read.  Returns a dict with the tangent of the solution ``x``,
+        ``u``, ``y``, ``rhs`` (dict q, r, c: the right-hand side t = dK z + dh the tangent
+        solve used) and ``status``.  Q and R enter through their symmetric parts; failed
+        problems and padding lanes get zero x, u, y."""
+        e = self.engine
+        unknown = set(tan) - set(_capi.LQR_INPUT_FIELDS)
+        if unknown:
+            raise ValueError(f"not an LQR input: {sorted(unknown)}")
+        dsol = self.alloc_output() if dsol is None else dsol
+        if rhs is None:
+            rhs = {k: e.empty(e.lqr_sizes[k]) for k in ("q", "r", "c")}
+        status = e.empty_int() if status is None else status
+        si, ss, st = _lqr_input_struct(inp), _lqr_output_struct(out), _lqr_input_struct(tan)
+        sr = _lqr_output_struct(dict(x=rhs["q"], u=rhs["r"], y=rhs["c"]))
+        sd = _lqr_output_struct(dsol)
+        e._check(lib.sipoc_lqr_jvp(e._handle, ctypes.byref(si), ctypes.byref(ss),
+                                   ctypes.byref(st), ctypes.byref(sr), ctypes.byref(sd),
+                                   status.data_ptr(), e.stream_ptr(stream)))
+        return dict(dsol, rhs=rhs, status=status)
+
     # -- optional FP32 mode (sipoc_lqr_factor_solve_f32; include/sipoc.h) -------------------
     @property
     def f32_supported(self) -> bool:
