@@ -822,63 +822,119 @@ riccati_backward_subwarp(LqrIn in, LqrOut out, int *status_out, double *store, d
     // ---- node k: compute_delta_sqrt + factor_F + compute_regularized_W --------
     // (lqr.cpp:475-529): V, v in registers -> W_k in shared memory and in the
     // store, v_k in shared memory and in the spill.
-    double sdo[SX], sdio[SX];
+    double sdo[SX], sdio[SX], sd[N];
 #pragma unroll
     for (int s = 0; s < SX; ++s) {
       sdo[s] = SM(S::rSd + xj[s]);
       sdio[s] = SM(S::rSdi + xj[s]);
     }
 #pragma unroll
+    for (int i = 0; i < N; ++i) sd[i] = SM(S::rSd + i);
+    // Own columns of F = I + D^1/2 V D^1/2 (rows >= 4 s).
+#pragma unroll
     for (int s = 0; s < SX; ++s)
 #pragma unroll
       for (int i = kGroup * s; i < N; ++i)
-        V[s][i] = SM(S::rSd + i) * V[s][i] * sdo[s] + (i == xj[s] ? 1.0 : 0.0);
+        V[s][i] = sd[i] * V[s][i] * sdo[s] + (i == xj[s] ? 1.0 : 0.0);
     __syncwarp();  // every lane is done with the exchange region (Lambda)
+    // F goes through the W rows (W_{k+1} is consumed), so the exchange rows can take the
+    // next stage's Q, M, R right away and the copy lands while F is factored.
+    if (k > 0) {
+      issue_qmr(true);
+      cp_async_commit();
+    }
 #pragma unroll
     for (int s = 0; s < SX; ++s) {
-#pragma unroll
-      for (int i = kGroup * s; i < N; ++i)
-        if (xok[s] && i >= xj[s]) SM(S::rX + qcol[s] + i) = V[s][i];
       if (SOLVE && xok[s]) {
         SM(S::rV + xj[s]) = vv[s];
         if (valid) stcs(vst + static_cast<int64_t>(xj[s]) * ld, vv[s]);
       }
     }
     if (SOLVE) vst -= static_cast<int64_t>(N) * ld;
-    __syncwarp();
     if (__ballot_sync(0xffffffffu, bad_delta) & group_mask) {
       if (status == SIPOC_FACTOR_SUCCESS) status = SIPOC_FACTOR_INVALID_DELTA;
     }
 
-    // Cholesky of F, replicated in the four lanes (registers only, no exchange).
+    // Cholesky of F = L L' (the diagonal of L keeps the pivots, dinv their rsqrt), blocked
+    // by kGroup columns: diagonal block b holds own column xj[b] of every lane.  Per block
+    // the lanes publish their columns of the block, every lane factors the diagonal block
+    // (replicated, so the rsqrt -> mul -> FMA chain needs no exchange), each lane solves
+    // its own rows xj[s] of the panel below and publishes them, and each lane applies the
+    // block's update to its own later columns.  Every entry takes its updates in ascending
+    // pivot order and the same scaling as the unblocked right-looking form, so L is the
+    // same to the bit; the trailing FMAs are split four ways instead of replicated.
     double L[tri(N)], dinv[N];
-#pragma unroll
-    for (int t = 0; t < tri(N); ++t) L[t] = SM(S::rX + t);
-    __syncwarp();  // every lane has read F: the exchange rows are free again
-    if (k > 0) {
-      issue_qmr(true);
-      cp_async_commit();
-    }
-    // Right-looking form: once column j is scaled, the trailing updates are independent
-    // FMAs, so the dependent chain per column is rsqrt -> mul -> one FMA.
     bool f_ok = true;
+    // One call per block with b a compile-time constant: a partial last block (n = 6) kept a
+    // plain unrolled loop from resolving the indices of L, which then went to local memory.
+    auto f_block = [&](auto b_tag) {
+      constexpr int b = decltype(b_tag)::value;
+      constexpr int j0 = kGroup * b, j1 = j0 + kGroup < N ? j0 + kGroup : N;
+      if (xok[b]) {
 #pragma unroll
-    for (int j = 0; j < N; ++j) {
-      const double x = L[pk(j, j, N)];
-      f_ok = f_ok && (x > 0.0);
-      const double d = rsqrt(x);
-      dinv[j] = d;
+        for (int i = j0; i < N; ++i)
+          if (i >= xj[b]) SM(S::rW + qcol[b] + i) = V[b][i];
+      }
+      __syncwarp();  // columns j0 .. j1 - 1 of F, all updates of earlier blocks applied
 #pragma unroll
-      for (int i = j + 1; i < N; ++i) L[pk(i, j, N)] *= d;
+      for (int j = j0; j < j1; ++j)
 #pragma unroll
-      for (int c = j + 1; c < N; ++c)
+        for (int i = j; i < j1; ++i) L[pk(i, j, N)] = SM(S::rW + pk(i, j, N));
 #pragma unroll
-        for (int i = c; i < N; ++i) L[pk(i, c, N)] -= L[pk(i, j, N)] * L[pk(c, j, N)];
-    }
+      for (int j = j0; j < j1; ++j) {
+        const double x = L[pk(j, j, N)];
+        f_ok = f_ok && (x > 0.0);
+        const double d = rsqrt(x);
+        dinv[j] = d;
+#pragma unroll
+        for (int i = j + 1; i < j1; ++i) L[pk(i, j, N)] *= d;
+#pragma unroll
+        for (int c = j + 1; c < j1; ++c)
+#pragma unroll
+          for (int i = c; i < j1; ++i) L[pk(i, c, N)] -= L[pk(i, j, N)] * L[pk(c, j, N)];
+      }
+      if constexpr (b + 1 < SX) {
+        // Own rows xj[s] of the panel: L(xj, j) for the block's columns j.
+        double lr[SX][kGroup];
+#pragma unroll
+        for (int s = b + 1; s < SX; ++s) {
+#pragma unroll
+          for (int j = j0; j < j1; ++j) {
+            double t = SM(S::rW + colbase(j, N) + xj[s]);
+#pragma unroll
+            for (int q = j0; q < j; ++q) t -= lr[s][q - j0] * L[pk(j, q, N)];
+            lr[s][j - j0] = t * dinv[j];
+          }
+          if (xok[s]) {
+#pragma unroll
+            for (int j = j0; j < j1; ++j) SM(S::rW + colbase(j, N) + xj[s]) = lr[s][j - j0];
+          }
+        }
+        __syncwarp();  // the panel of the block is solved
+#pragma unroll
+        for (int j = j0; j < j1; ++j)
+#pragma unroll
+          for (int i = j1; i < N; ++i) L[pk(i, j, N)] = SM(S::rW + pk(i, j, N));
+#pragma unroll
+        for (int s = b + 1; s < SX; ++s)
+#pragma unroll
+          for (int j = j0; j < j1; ++j)
+#pragma unroll
+            for (int i = kGroup * s; i < N; ++i) V[s][i] -= L[pk(i, j, N)] * lr[s][j - j0];
+      }
+    };
+    f_block(std::integral_constant<int, 0>{});
+    if constexpr (SX > 1) f_block(std::integral_constant<int, 1>{});
+    if constexpr (SX > 2) f_block(std::integral_constant<int, 2>{});
+    if constexpr (SX > 3) f_block(std::integral_constant<int, 3>{});
+    __syncwarp();  // every lane has read F: the W rows take W_k
     if (!f_ok && status == SIPOC_FACTOR_SUCCESS) status = SIPOC_FACTOR_F_FACTORIZATION_FAILURE;
     // Own columns of F^-1 = L^-T L^-1: forward substitution on e_xj, then backward
     // substitution, both against the lane's register copy of L (no exchange).
     // W = D^-1/2 (I - F^-1) D^-1/2, rows >= 4 s of the own columns.
+    double sdi[N];
+#pragma unroll
+    for (int i = 0; i < N; ++i) sdi[i] = SM(S::rSdi + i);
 #pragma unroll
     for (int s = 0; s < SX; ++s) {
       // Column-oriented (axpy) substitutions: each solved entry immediately updates
@@ -901,7 +957,7 @@ riccati_backward_subwarp(LqrIn in, LqrOut out, int *status_out, double *store, d
       double *dst = Wst + static_cast<int64_t>(qcol[s] + kGroup * s) * ld;
 #pragma unroll
       for (int i = kGroup * s; i < N; ++i) {
-        const double w = SM(S::rSdi + i) * ((i == xj[s] ? 1.0 : 0.0) - y[i]) * sdio[s];
+        const double w = sdi[i] * ((i == xj[s] ? 1.0 : 0.0) - y[i]) * sdio[s];
         if (xok[s] && i >= xj[s]) {
           if constexpr (PACKW) {
             SM(S::rW + qcol[s] + i) = w;
