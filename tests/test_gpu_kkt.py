@@ -293,29 +293,6 @@ def test_host_buffer_entry_points():
     assert (np.linalg.norm(prod - rhs, axis=1) / np.linalg.norm(rhs, axis=1)).max() < 1e-9
 
 
-def test_fused_kkt_solve_path_large_batch():
-    """Above the dispatch threshold the uniform-chain solve runs the fused kernels (rhs
-    build inside the affine sweep, dual recovery inside the rollout); same parity bar."""
-    n, m, T, batch = 4, 1, 6, 32768 + 5
-    s = _uniform_kkt_structure(n, m, T)
-    model, w, r1, r2, r3, rhs = pg.newton_kkt_batch(s, batch, seed=21, r2_max=1e9)
-    sample = np.r_[0:64, batch - 64:batch]
-    sub = lambda a: a[sample]
-    ref = pyoracle.kkt_factor_solve(s, {k: sub(v) for k, v in model.items()}, sub(w), sub(r1),
-                                    sub(r2), sub(r3), sub(rhs))
-    gpu, cp, dev = _gpu_kkt(s, model, w, r1, r2, r3, rhs)
-    assert "generic" not in cp.engine.kernel_variant
-    good = ref["ok"] == 1
-    assert good.sum() >= sample.size - 4
-    assert (gpu["ok"][sample] == ref["ok"]).all()
-    assert rel_err(gpu["sol"][sample][good], ref["sol"][good]).max() < 1e-9
-    ref_res = _oracle_residual(s, {k: sub(v) for k, v in model.items()}, sub(w), sub(r1), sub(r2),
-                               sub(r3), ref["sol"], sub(rhs))
-    scale = np.linalg.norm(rhs, axis=1)[sample]
-    assert (gpu["residual"][sample][good] / scale[good]).max() <= \
-        10.0 * (ref_res[good] / scale[good]).max()
-
-
 @pytest.mark.parametrize("uniform", [True, False])
 def test_captured_step_replays_bit_exact(uniform):
     """CallbackProvider.capture_step: the CUDA-graph replay of factor + solve + residual
