@@ -308,6 +308,38 @@ sipoc_error sipoc_lqr_jvp(sipoc_engine *engine, const sipoc_lqr_input *in,
                           const sipoc_lqr_output *rhs, const sipoc_lqr_output *dsol,
                           int *status, void *stream);
 
+/* ---- feedback policy of the LQR solve --------------------------------------------------
+ * sipoc_lqr_factor_solve_policy does exactly what sipoc_lqr_factor_solve does, on the same
+ * plan (x, u, y and status are bitwise the same, and the handle's kept factorization is
+ * replaced the same way), then writes the policy the Riccati recursion computed, per problem:
+ *   u_e = K_e x_p + k_e   (p: parent node of edge e)       y_i = V_i x_i + v_i
+ * These are the reference's K, k, V, v after factor_with_status + solve (lqr.cpp:658,
+ * :707-719, :744, :785-794).  V is the Hessian of the cost-to-go BEFORE the delta
+ * regularization, so y_i = v_i + V_i x_i holds for the solution.  Layouts, per problem, in the
+ * flat index of this header (each array reuses the element count of an input):
+ *   K : per edge, m_e x n_p column-major (the element count of M)
+ *   k : per edge, m_e                     (the element count of r)
+ *   V : per node, n_i x n_i, both triangles, exactly symmetric on the shape-specialised
+ *       plans (the element count of Q)
+ *   v : per node, n_i                     (the element count of q)
+ *   policy : required; any of its four arrays may be NULL, and is then neither computed nor
+ *            written (K, k alone do not pay for V, which the plans that keep F^-1 instead
+ *            rebuild per edge from Q, M, A, B, delta, F^-1 and K).
+ *   status : as for sipoc_lqr_factor_solve, or NULL (an engine-owned buffer is used).
+ * Every requested array is written in full: zeros in problems whose status != 0 and in the
+ * padding lanes batch <= b < batch_stride.  FP64, device engine layout only, 16-byte aligned
+ * arrays; the call only enqueues work on `stream` and can be recorded in a graph once it has
+ * run eagerly (its workspaces are sized on the first call).  On the parallel-in-time plan a
+ * node shared by two segments takes its values from the later one (node s L from segment s),
+ * and the last node from the last segment. */
+typedef struct sipoc_lqr_policy {
+  double *K, *k, *V, *v;
+} sipoc_lqr_policy;
+sipoc_error sipoc_lqr_factor_solve_policy(sipoc_engine *engine, const sipoc_lqr_input *in,
+                                          const sipoc_lqr_output *out,
+                                          const sipoc_lqr_policy *policy, int *status,
+                                          void *stream);
+
 /* ---- layout conversion (device <-> device) ------------------------------ */
 /* src: problem-major [batch][size]; dst: engine layout [size][batch_stride]. */
 sipoc_error sipoc_pack(sipoc_engine *engine, const double *src, double *dst,

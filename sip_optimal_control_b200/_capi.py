@@ -75,6 +75,15 @@ class LqrGrad(ctypes.Structure):
     _fields_ = [(k, c_void_p) for k in LQR_INPUT_FIELDS]
 
 
+# sipoc_lqr_policy: feedback gains K, k and cost-to-go V, v; the element counts of M, r, Q, q
+LQR_POLICY_FIELDS = ("K", "k", "V", "v")
+LQR_POLICY_SIZE_OF = dict(K="M", k="r", V="Q", v="q")
+
+
+class LqrPolicy(ctypes.Structure):
+    _fields_ = [(k, c_void_p) for k in LQR_POLICY_FIELDS]
+
+
 KKT_THETA_FIELDS = ("node_hxt", "node_jct", "node_jgt", "node_htt", "edge_hxt", "edge_hut",
                     "edge_dynt", "edge_jct", "edge_jgt", "edge_htt")
 
@@ -185,6 +194,7 @@ def _load() -> ctypes.CDLL:
     lib.sipoc_lqr_vjp.argtypes = [E, LI, LO, ctypes.POINTER(LqrCotangent), LO,
                                   ctypes.POINTER(LqrGrad), P, P]
     lib.sipoc_lqr_jvp.argtypes = [E, LI, LO, LI, LO, LO, P, P]
+    lib.sipoc_lqr_factor_solve_policy.argtypes = [E, LI, LO, ctypes.POINTER(LqrPolicy), P, P]
     lib.sipoc_status_stats.argtypes = [E, P, P, P]
     lib.sipoc_pack.argtypes = [E, P, P, ctypes.c_int64, P]
     lib.sipoc_unpack.argtypes = [E, P, P, ctypes.c_int64, P]

@@ -18,6 +18,7 @@
 #include "jvp.cuh"
 #include "kkt_vjp.cuh"
 #include "lqr_vjp.cuh"
+#include "policy.cuh"
 #include "scan.cuh"
 #include "model_scatter.cuh"
 #include "riccati_f32.cuh"
@@ -107,6 +108,7 @@ struct sipoc_engine {
   double *f64t_store = nullptr;
   double *h_packed = nullptr;  // packed-symmetric host entry: Q / R triangles before expansion
   int *vjp_status = nullptr;   // status / ok of sipoc_*_vjp / _jvp when the caller passes none (lazy)
+  double *policy_V = nullptr;  // V rebuilt in a padded plan's shape, before extraction (lazy)
 
   // Parallel-in-time factor + solve (scan.cu): long uniform chains, small batches.
   struct Scan {
@@ -1343,6 +1345,107 @@ sipoc_error sipoc_lqr_jvp(sipoc_engine *e, const sipoc_lqr_input *in,
   }
   e->launches += 3;
   return check_launch(e, "lqr_jvp zero pass");
+}
+
+// The policy of the factor + solve that has just run (policy.cuh).  `scan`: it ran parallel
+// in time, on the per-segment stores.  Generic and strict plans keep V; the others keep
+// F^-1, from which V is rebuilt; padded plans are exported in their own shape and the
+// leading blocks extracted.
+static sipoc_error lqr_policy_export(sipoc_engine *e, const LqrIn &caller_in, const LqrPolicy &pol,
+                                     const int *status, bool scan, cudaStream_t s) {
+  const HostStructure &h = e->hs;
+  auto gather = [&](PolicyArray which, const PolicySrc &src, double *dst) {
+    if (dst == nullptr) return;
+    ProfScope ps(&e->prof, "policy_gather_kernel", s);
+    launch_policy_gather(e->dt, which, src, dst, status, e->batch, e->ld, s);
+    e->launches += 1;
+  };
+  if (!scan && e->factored == sipoc_engine::Factored::GENERIC) {
+    PolicySrc src;
+    src.same_as_out = true;
+    src.p = e->gws.K;
+    gather(PolicyArray::K, src, pol.K);
+    src.p = e->gws.k;
+    gather(PolicyArray::k, src, pol.k);
+    src.p = e->gws.V;
+    gather(PolicyArray::V, src, pol.V);
+    src.p = e->gws.v;
+    gather(PolicyArray::v, src, pol.v);
+    return check_launch(e, "lqr policy export");
+  }
+  const FastPlan *plan = e->fast;
+  const int n = plan->n, m = plan->m;
+  const bool strict = plan == select_strict_plan(n, m) || plan == select_strict_tree_plan(n, m);
+  const PolicyStore kind = plan->problem_major_inputs ? PolicyStore::CTA
+                           : strict                   ? PolicyStore::STRICT
+                                                      : PolicyStore::FAST;
+  const int T = scan ? e->scan.L : h.E;
+  PolicySources src = policy_sources(kind, n, m, T, scan ? e->scan.store : e->fast_store,
+                                     scan ? e->scan.scratch : e->fast_scratch);
+  if (scan) {
+    for (PolicySrc *p : {&src.K, &src.k, &src.v, &src.V_or_P}) {
+      p->seg_len = e->scan.L;
+      p->segs = e->scan.S;
+    }
+    src.K.seg_stride = src.V_or_P.seg_stride = plan->store_elems(T);
+    src.k.seg_stride = src.v.seg_stride = plan->scratch_elems(T);
+  }
+  gather(PolicyArray::K, src.K, pol.K);
+  gather(PolicyArray::k, src.k, pol.k);
+  gather(PolicyArray::v, src.v, pol.v);
+  if (pol.V != nullptr && kind == PolicyStore::STRICT) {
+    gather(PolicyArray::V, src.V_or_P, pol.V);
+  } else if (pol.V != nullptr) {
+    // the arrays the plan ran on: its padded copies on padded plans
+    const LqrIn in = e->padded ? LqrIn{e->pad_in[0], e->pad_in[1], e->pad_in[2],
+                                       e->pad_in[3], e->pad_in[4], e->pad_in[5],
+                                       e->pad_in[6], e->pad_in[7], e->pad_in[8]}
+                               : caller_in;
+    double *V = pol.V;
+    if (e->padded) {
+      if (e->policy_V == nullptr) {
+        const sipoc_error rc = alloc_doubles(e, &e->policy_V, int64_t(h.E + 1) * n * n);
+        if (rc != SIPOC_OK) return rc;
+      }
+      V = e->policy_V;
+    }
+    bool ok;
+    {
+      ProfScope ps(&e->prof, "policy_rebuild_v_kernel", s);
+      ok = launch_policy_rebuild_v(n, m, in, src.V_or_P, src.K, V, status, h.E, e->batch, e->ld, s);
+    }
+    if (!ok) return fail(e, SIPOC_UNSUPPORTED, "no V rebuild kernel for the plan's shape");
+    e->launches += 1;
+    if (e->padded) {
+      PolicySrc pad;
+      pad.p = e->policy_V;
+      pad.rows = n;
+      pad.block = int64_t(n) * n;
+      gather(PolicyArray::V, pad, pol.V);
+    }
+  }
+  return check_launch(e, "lqr policy export");
+}
+
+sipoc_error sipoc_lqr_factor_solve_policy(sipoc_engine *e, const sipoc_lqr_input *in,
+                                          const sipoc_lqr_output *out,
+                                          const sipoc_lqr_policy *policy, int *status,
+                                          void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (null_in(in, true, true) || out == nullptr || !out->x || !out->u || !out->y ||
+      policy == nullptr)
+    return fail(e, SIPOC_INVALID_ARGUMENT, "NULL LQR input / output / policy");
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  sipoc_error rc;
+  if ((rc = default_vjp_status(e, &status)) != SIPOC_OK) return rc;
+  const LqrIn cin = to_in(in);
+  const bool scan = e->scan.enabled && use_fast(e, cin);  // the branch lqr_factor_solve_core takes
+  if ((rc = lqr_factor_solve_core(e, cin, LqrOut{out->x, out->u, out->y}, status, s)) != SIPOC_OK)
+    return rc;
+  const LqrPolicy pol{policy->K, policy->k, policy->V, policy->v};
+  if (!pol.K && !pol.k && !pol.V && !pol.v) return SIPOC_OK;
+  return lqr_policy_export(e, cin, pol, status, scan, s);
 }
 
 sipoc_error sipoc_status_stats(sipoc_engine *e, const int *status, double *stats,

@@ -484,4 +484,13 @@ bool BatchedLQR::factor_solve(const DeviceInput &in, const DeviceOutput &out, in
          sipoc_lqr_factor_solve(engine_, &a, &o, status, stream) == SIPOC_OK;
 }
 
+bool BatchedLQR::factor_solve_policy(const DeviceInput &in, const DeviceOutput &out,
+                                     const DevicePolicy &policy, int *status, void *stream) {
+  const sipoc_lqr_input a = to_abi(in);
+  const sipoc_lqr_output o{out.x, out.u, out.y};
+  const sipoc_lqr_policy p{policy.K, policy.k, policy.V, policy.v};
+  return engine_ != nullptr &&
+         sipoc_lqr_factor_solve_policy(engine_, &a, &o, &p, status, stream) == SIPOC_OK;
+}
+
 }  // namespace sip::optimal_control

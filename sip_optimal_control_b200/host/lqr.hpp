@@ -227,6 +227,13 @@ class BatchedLQR {
   bool solve(const DeviceInput &in, const DeviceOutput &out, void *stream = nullptr);
   bool factor_solve(const DeviceInput &in, const DeviceOutput &out, int *status,
                     void *stream = nullptr);
+  // factor_solve, then the feedback policy u_e = K_e x_parent + k_e, y_i = V_i x_i + v_i of
+  // every problem (sipoc_lqr_factor_solve_policy); a nullptr array is not computed.
+  struct DevicePolicy {
+    double *K, *k, *V, *v;
+  };
+  bool factor_solve_policy(const DeviceInput &in, const DeviceOutput &out,
+                           const DevicePolicy &policy, int *status, void *stream = nullptr);
 
  private:
   sipoc_engine *engine_ = nullptr;

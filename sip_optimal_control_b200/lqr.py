@@ -386,6 +386,40 @@ class LQR:
                                             status.data_ptr(), e.stream_ptr(stream)))
         return status
 
+    def factor_solve_policy(self, inp: dict, out: dict, want=None, policy=None, status=None,
+                            stream=None) -> dict:
+        """``factor_solve`` that also returns the feedback policy of the solve
+        (sipoc_lqr_factor_solve_policy; include/sipoc.h).
+
+        x, u, y and the status are bitwise those of ``factor_solve``.  ``want`` is a subset of
+        ``{"K", "k", "V", "v"}`` (default: all four); the others are neither computed nor
+        written.  Returns a dict with one engine-layout tensor per wanted name -- per edge
+        ``u_e = K_e x_parent(e) + k_e`` (K: m_e x n_parent column-major, the element count of
+        M; k: that of r), per node ``y_i = V_i x_i + v_i`` (V: n_i x n_i, that of Q; v: that
+        of q) -- and ``status``.  ``policy`` may supply the output tensors.  Failed problems
+        and padding lanes get zeros.  The outputs are plain tensors: autograd does not
+        differentiate through them."""
+        if self.traversal_status_ != FactorStatus.SUCCESS:
+            return dict(status=self._invalid())
+        e = self.engine
+        want = set(_capi.LQR_POLICY_FIELDS if want is None else want)
+        unknown = want - set(_capi.LQR_POLICY_FIELDS)
+        if unknown:
+            raise ValueError(f"not a policy array: {sorted(unknown)}")
+        given = {} if policy is None else policy
+        arrays = {k: given[k] if k in given else e.empty(e.lqr_sizes[_capi.LQR_POLICY_SIZE_OF[k]])
+                  for k in _capi.LQR_POLICY_FIELDS if k in want}
+        status = e.empty_int() if status is None else status
+        si, so = _lqr_input_struct(inp), _lqr_output_struct(out)
+        sp = _capi.LqrPolicy()
+        for k in _capi.LQR_POLICY_FIELDS:
+            setattr(sp, k, arrays[k].data_ptr() if k in arrays else None)
+        e._check(lib.sipoc_lqr_factor_solve_policy(e._handle, ctypes.byref(si), ctypes.byref(so),
+                                                   ctypes.byref(sp), status.data_ptr(),
+                                                   e.stream_ptr(stream)))
+        arrays["status"] = status
+        return arrays
+
     def vjp(self, inp: dict, out: dict, cot: dict, want=None, adjoint=None, status=None,
             stream=None) -> dict:
         """Reverse-mode derivative of ``factor_solve`` (sipoc_lqr_vjp; include/sipoc.h).
