@@ -340,6 +340,37 @@ sipoc_error sipoc_lqr_factor_solve_policy(sipoc_engine *engine, const sipoc_lqr_
                                           const sipoc_lqr_policy *policy, int *status,
                                           void *stream);
 
+/* ---- reverse-mode derivative of the feedback policy -------------------------------------
+ * For cotangents (Kb, kb, Vb, vb) = dL/d(K, k, V, v) of the policy sipoc_lqr_factor_solve_policy
+ * returned, sipoc_lqr_policy_vjp writes the gradient of L with respect to the inputs, per
+ * problem, in each input array's own layout.  It is the adjoint of the Riccati recursion, one
+ * sweep from the root to the leaves: K_e and V_i are sensitivities of tail subproblems, not
+ * functions of one solution, so they have no cheaper route through sipoc_lqr_vjp.  Per edge
+ * the recursion is recomputed from the inputs and the forward's V, v (W_c from the Cholesky
+ * factor of I + D^1/2 V_c D^1/2, K and k from that of G), so the call keeps no state from the
+ * forward and works the same whichever plan ran it.  K and V do not depend on q, r, c: with
+ * only Kb and Vb given, the gradients of q, r, c are exactly zero.
+ *   in     : R, M, r, A, B, c, delta of the forward are read; Q and q are not and may be NULL.
+ *   V, v   : the forward's policy arrays, required.  Only the lower triangle of V is read.
+ *   status : the forward's per-problem FactorStatus, required.
+ *   cot    : required; any of its four arrays may be NULL, which is bitwise the same as zeros.
+ *   grad   : required; any of its arrays may be NULL, and is then neither computed nor
+ *            written.  Q and R get the gradient with respect to the SYMMETRIC matrices (the
+ *            same values in both triangles), as for sipoc_lqr_vjp.  The root's c and delta get
+ *            zero gradient.
+ * Every requested gradient array is written in full: zeros in problems whose status != 0 and
+ * in the padding lanes batch <= b < batch_stride.  Any structure sipoc_lqr_factor_solve_policy
+ * accepts.  FP64, engine layout, 16-byte aligned arrays.  Trees and shapes without a
+ * specialised kernel use an engine-owned workspace sized on the first call, so the call can
+ * be recorded in a graph once it has run eagerly. */
+typedef struct sipoc_lqr_policy_cotangent {
+  const double *K, *k, *V, *v;
+} sipoc_lqr_policy_cotangent;
+sipoc_error sipoc_lqr_policy_vjp(sipoc_engine *engine, const sipoc_lqr_input *in,
+                                 const double *V, const double *v, const int *status,
+                                 const sipoc_lqr_policy_cotangent *cot,
+                                 const sipoc_lqr_grad *grad, void *stream);
+
 /* ---- layout conversion (device <-> device) ------------------------------ */
 /* src: problem-major [batch][size]; dst: engine layout [size][batch_stride]. */
 sipoc_error sipoc_pack(sipoc_engine *engine, const double *src, double *dst,

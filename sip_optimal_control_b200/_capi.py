@@ -84,6 +84,11 @@ class LqrPolicy(ctypes.Structure):
     _fields_ = [(k, c_void_p) for k in LQR_POLICY_FIELDS]
 
 
+# sipoc_lqr_policy_cotangent: dL/d(K, k, V, v); any may be NULL (zeros)
+class LqrPolicyCotangent(ctypes.Structure):
+    _fields_ = [(k, c_void_p) for k in LQR_POLICY_FIELDS]
+
+
 KKT_THETA_FIELDS = ("node_hxt", "node_jct", "node_jgt", "node_htt", "edge_hxt", "edge_hut",
                     "edge_dynt", "edge_jct", "edge_jgt", "edge_htt")
 
@@ -195,6 +200,8 @@ def _load() -> ctypes.CDLL:
                                   ctypes.POINTER(LqrGrad), P, P]
     lib.sipoc_lqr_jvp.argtypes = [E, LI, LO, LI, LO, LO, P, P]
     lib.sipoc_lqr_factor_solve_policy.argtypes = [E, LI, LO, ctypes.POINTER(LqrPolicy), P, P]
+    lib.sipoc_lqr_policy_vjp.argtypes = [E, LI, P, P, P, ctypes.POINTER(LqrPolicyCotangent),
+                                         ctypes.POINTER(LqrGrad), P]
     lib.sipoc_status_stats.argtypes = [E, P, P, P]
     lib.sipoc_pack.argtypes = [E, P, P, ctypes.c_int64, P]
     lib.sipoc_unpack.argtypes = [E, P, P, ctypes.c_int64, P]

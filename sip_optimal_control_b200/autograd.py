@@ -13,6 +13,13 @@ Conventions (include/sipoc.h, sipoc_lqr_vjp):
 - Problems whose factorization fails (status != 0) and the padding lanes
   batch <= b < batch_stride get zero gradients.
 
+``factor_solve_policy(lqr, inp)`` runs ``LQR.factor_solve_policy`` and returns
+``(x, u, y, K, k, V, v, status)``: the solution and the feedback policy
+``u_e = K_e x_parent(e) + k_e``, ``y_i = V_i x_i + v_i``.  Its backward runs ``sipoc_lqr_vjp``
+for the cotangents of x, u, y and ``sipoc_lqr_policy_vjp`` (the adjoint Riccati sweep) for
+those of K, k, V, v, each only when one of its cotangents is given, and sums the two.  It has
+no forward mode: ``forward_ad`` and ``torch.func.jvp`` through it raise torch's own error.
+
 ``kkt_factor_solve(cp, model, w, r1, r2, r3, b)`` does the same for the Newton-KKT solve
 (``CallbackProvider.factor`` + ``solve``) and returns ``(sol, ok)``; sol carries gradients
 back to the model blocks (theta blocks included), w, r1, r2, r3 and b through
@@ -20,7 +27,7 @@ back to the model blocks (theta blocks included), w, r1, r2, r3 and b through
 symmetric Hessian blocks (node_hxx, edge_hxx, edge_huu, node_htt, edge_htt) get the
 symmetric gradient, and problems with ok == 0 and the padding lanes get zeros.
 
-Both Functions also differentiate in forward mode (``torch.autograd.forward_ad`` dual tensors,
+``factor_solve`` and ``kkt_factor_solve`` also differentiate in forward mode (``torch.autograd.forward_ad`` dual tensors,
 ``torch.func.jvp``, ``gradcheck(..., check_forward_ad=True)``): the tangent of the solution is
 one more solve of the same system whose right-hand side the tangents of the inputs build
 (``sipoc_lqr_jvp`` / ``sipoc_kkt_jvp``).  Absent tangents cost nothing; the symmetric blocks
@@ -96,6 +103,50 @@ def factor_solve(lqr, inp: dict):
     differentiable.  ``inp`` holds float64 CUDA tensors in the engine layout
     ``[size, batch_stride]`` (``LQR.alloc_input`` / ``LQR.pack_input``)."""
     return _FactorSolve.apply(lqr, *(inp[k] for k in LQR_INPUT_FIELDS))
+
+
+class _FactorSolvePolicy(torch.autograd.Function):
+    @staticmethod
+    def forward(lqr, *arrays):
+        inp = {k: a.contiguous() for k, a in zip(LQR_INPUT_FIELDS, arrays)}
+        out = lqr.alloc_output()
+        pol = lqr.factor_solve_policy(inp, out)  # all four: the backward needs V and v
+        return out["x"], out["u"], out["y"], pol["K"], pol["k"], pol["V"], pol["v"], pol["status"]
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        lqr, *arrays = inputs
+        x, u, y, _K, _k, V, v, status = output
+        ctx.lqr = lqr
+        ctx.save_for_backward(*arrays, x, u, y, V, v, status)
+        ctx.mark_non_differentiable(status)
+        ctx.set_materialize_grads(False)  # an absent cotangent skips its half of the backward
+
+    @staticmethod
+    def backward(ctx, gx, gu, gy, gK, gk, gV, gv, _gstatus):
+        saved = [a.contiguous() for a in ctx.saved_tensors]
+        n = len(LQR_INPUT_FIELDS)
+        inp = dict(zip(LQR_INPUT_FIELDS, saved[:n]))
+        x, u, y, V, v, status = saved[n:]
+        want = {k for k, need in zip(LQR_INPUT_FIELDS, ctx.needs_input_grad[1:]) if need}
+        total = {}
+        if want and any(g is not None for g in (gx, gu, gy)):
+            cot = {k: torch.zeros_like(ref) if g is None else g.contiguous()
+                   for k, g, ref in (("x", gx, x), ("u", gu, u), ("y", gy, y))}
+            total = {k: g for k, g in ctx.lqr.vjp(inp, dict(x=x, u=u, y=y), cot, want=want).items()
+                     if k in want}
+        if want and any(g is not None for g in (gK, gk, gV, gv)):
+            cot = {k: g.contiguous() for k, g in (("K", gK), ("k", gk), ("V", gV), ("v", gv))
+                   if g is not None}
+            pg = ctx.lqr.policy_vjp(inp, dict(V=V, v=v), status, cot, want=want)
+            total = {k: total[k] + pg[k] if k in total else pg[k] for k in pg}
+        return (None,) + tuple(total.get(k) for k in LQR_INPUT_FIELDS)
+
+
+def factor_solve_policy(lqr, inp: dict):
+    """Differentiable ``lqr.factor_solve_policy``: returns (x, u, y, K, k, V, v, status),
+    status not differentiable.  ``inp`` as for ``factor_solve``.  Reverse mode only."""
+    return _FactorSolvePolicy.apply(lqr, *(inp[k] for k in LQR_INPUT_FIELDS))
 
 
 _KKT_VECTORS = ("w", "r1", "r2", "r3", "b")

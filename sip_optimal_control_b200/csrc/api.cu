@@ -19,6 +19,7 @@
 #include "kkt_vjp.cuh"
 #include "lqr_vjp.cuh"
 #include "policy.cuh"
+#include "policy_vjp.cuh"
 #include "scan.cuh"
 #include "model_scatter.cuh"
 #include "riccati_f32.cuh"
@@ -109,6 +110,7 @@ struct sipoc_engine {
   double *h_packed = nullptr;  // packed-symmetric host entry: Q / R triangles before expansion
   int *vjp_status = nullptr;   // status / ok of sipoc_*_vjp / _jvp when the caller passes none (lazy)
   double *policy_V = nullptr;  // V rebuilt in a padded plan's shape, before extraction (lazy)
+  double *policy_vjp_ws = nullptr;  // edge scratch and per-node Vb, vb of the generic policy VJP (lazy)
 
   // Parallel-in-time factor + solve (scan.cu): long uniform chains, small batches.
   struct Scan {
@@ -1446,6 +1448,43 @@ sipoc_error sipoc_lqr_factor_solve_policy(sipoc_engine *e, const sipoc_lqr_input
   const LqrPolicy pol{policy->K, policy->k, policy->V, policy->v};
   if (!pol.K && !pol.k && !pol.V && !pol.v) return SIPOC_OK;
   return lqr_policy_export(e, cin, pol, status, scan, s);
+}
+
+// Reverse mode of the policy (policy_vjp.cuh): the adjoint Riccati sweep, root to leaves.
+// Uniform chains at the shapes of the thread and four-lane plans run the shape-specialised
+// kernel, every other structure the generic one; the choice depends on the structure only.
+sipoc_error sipoc_lqr_policy_vjp(sipoc_engine *e, const sipoc_lqr_input *in, const double *V,
+                                 const double *v, const int *status,
+                                 const sipoc_lqr_policy_cotangent *cot,
+                                 const sipoc_lqr_grad *grad, void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (in == nullptr || !in->M || !in->R || !in->r || !in->A || !in->B || !in->c || !in->delta ||
+      V == nullptr || v == nullptr || status == nullptr || cot == nullptr || grad == nullptr)
+    return fail(e, SIPOC_INVALID_ARGUMENT,
+                "NULL LQR input / policy V, v / status / cotangent / grad");
+  const LqrGrad g{grad->Q, grad->M, grad->R, grad->q, grad->r, grad->A, grad->B, grad->c,
+                  grad->delta};
+  if (!g.Q && !g.M && !g.R && !g.q && !g.r && !g.A && !g.B && !g.c && !g.delta) return SIPOC_OK;
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const HostStructure &h = e->hs;
+  const PolicyVjpIn pin{to_in(in), V, v};
+  const LqrPolicyCot pc{cot->K, cot->k, cot->V, cot->v};
+  if (h.is_chain && h.is_uniform && h.E >= 1 && policy_vjp_chain_shape(h.n[0], h.m[0])) {
+    ProfScope ps(&e->prof, "policy_vjp_kernel", s);
+    launch_policy_vjp_chain(h.n[0], h.m[0], h.E, pin, pc, g, status, e->batch, e->ld, s);
+  } else {
+    if (e->policy_vjp_ws == nullptr) {
+      const sipoc_error rc =
+          alloc_doubles(e, &e->policy_vjp_ws,
+                        policy_vjp_scratch_elems(h.max_n, h.max_m) + h.nn_off[h.N] + h.n_off[h.N]);
+      if (rc != SIPOC_OK) return rc;
+    }
+    ProfScope ps(&e->prof, "policy_vjp_generic_kernel", s);
+    launch_policy_vjp_generic(e->dt, h, pin, pc, g, e->policy_vjp_ws, status, e->batch, e->ld, s);
+  }
+  e->launches += 1;
+  return check_launch(e, "lqr policy vjp");
 }
 
 sipoc_error sipoc_status_stats(sipoc_engine *e, const int *status, double *stats,

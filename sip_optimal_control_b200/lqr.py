@@ -397,8 +397,8 @@ class LQR:
         ``u_e = K_e x_parent(e) + k_e`` (K: m_e x n_parent column-major, the element count of
         M; k: that of r), per node ``y_i = V_i x_i + v_i`` (V: n_i x n_i, that of Q; v: that
         of q) -- and ``status``.  ``policy`` may supply the output tensors.  Failed problems
-        and padding lanes get zeros.  The outputs are plain tensors: autograd does not
-        differentiate through them."""
+        and padding lanes get zeros.  The outputs are plain tensors; the differentiable variant
+        is ``autograd.factor_solve_policy``, whose backward runs ``policy_vjp``."""
         if self.traversal_status_ != FactorStatus.SUCCESS:
             return dict(status=self._invalid())
         e = self.engine
@@ -450,6 +450,43 @@ class LQR:
                                    status.data_ptr(), e.stream_ptr(stream)))
         grads["adjoint"] = adjoint
         grads["status"] = status
+        return grads
+
+    def policy_vjp(self, inp: dict, policy: dict, status, cot: dict, want=None, grad=None,
+                   stream=None) -> dict:
+        """Reverse-mode derivative of the policy of ``factor_solve_policy``
+        (sipoc_lqr_policy_vjp; include/sipoc.h).
+
+        ``inp`` holds the forward's inputs (Q and q are not read), ``policy`` its ``V`` and
+        ``v`` (both required: the adjoint sweep recomputes W, G, K and k from them), ``status``
+        its per-problem FactorStatus.  ``cot`` holds dL/dK, dL/dk, dL/dV, dL/dv for any subset
+        of the four names (engine layout); an absent name is a zero cotangent and is not read.
+        ``want`` is the set of input names to differentiate (default: all nine); the others are
+        neither computed nor written.  ``grad`` may supply the output tensors.  Returns a dict
+        with one engine-layout gradient tensor per wanted name.  Q and R get the symmetric
+        gradient; failed problems and padding lanes get zeros."""
+        e = self.engine
+        want = set(_capi.LQR_INPUT_FIELDS if want is None else want)
+        unknown = want - set(_capi.LQR_INPUT_FIELDS)
+        if unknown:
+            raise ValueError(f"not an LQR input: {sorted(unknown)}")
+        unknown = set(cot) - set(_capi.LQR_POLICY_FIELDS)
+        if unknown:
+            raise ValueError(f"not a policy array: {sorted(unknown)}")
+        given = {} if grad is None else grad
+        grads = {k: given[k] if k in given else e.empty(e.lqr_sizes[k])
+                 for k in _capi.LQR_INPUT_FIELDS if k in want}
+        si = _lqr_input_struct(inp)
+        sc = _capi.LqrPolicyCotangent()
+        for k in _capi.LQR_POLICY_FIELDS:
+            setattr(sc, k, cot[k].data_ptr() if cot.get(k) is not None else None)
+        sg = _capi.LqrGrad()
+        for k in _capi.LQR_INPUT_FIELDS:
+            setattr(sg, k, grads[k].data_ptr() if k in grads else None)
+        e._check(lib.sipoc_lqr_policy_vjp(e._handle, ctypes.byref(si), policy["V"].data_ptr(),
+                                          policy["v"].data_ptr(), status.data_ptr(),
+                                          ctypes.byref(sc), ctypes.byref(sg),
+                                          e.stream_ptr(stream)))
         return grads
 
     def jvp(self, inp: dict, out: dict, tan: dict, dsol=None, rhs=None, status=None,
