@@ -371,6 +371,42 @@ sipoc_error sipoc_lqr_policy_vjp(sipoc_engine *engine, const sipoc_lqr_input *in
                                  const sipoc_lqr_policy_cotangent *cot,
                                  const sipoc_lqr_grad *grad, void *stream);
 
+/* ---- forward-mode derivative of the feedback policy -------------------------------------
+ * For tangents (dQ, dM, dR, dq, dr, dA, dB, dc, ddelta) of the inputs, sipoc_lqr_policy_jvp
+ * writes the tangents (dK, dk, dV, dv) of the policy sipoc_lqr_factor_solve_policy returned.
+ * It is the tangent of the Riccati recursion, one sweep from the leaves to the root, the
+ * direction of the factorization: each edge needs only its child's dV, dv.  Per edge
+ * e = (p -> c), with the primal recomputed as sipoc_lqr_policy_vjp does (D = diag delta_c):
+ *   P = (I + D^1/2 V_c D^1/2)^-1   W = D^-1/2 (I - P) D^-1/2   S = (I + D V_c)^-1
+ *   G = R + B'WB   Y = WA   H = M' + B'Y   K = -G^-1 H
+ *   f = delta_c .* v_c - c_c   g = v_c - W f   h = r + B'g   k = -G^-1 h
+ *   dW = S' dV_c S - W dD W   dG = sym(dR) + dB'WB + B'W dB + B' dW B
+ *   dY = dW A + W dA   dH = dM' + dB'Y + B' dY   dK = -G^-1 (dH + dG K)
+ *   df = ddelta_c .* v_c + delta_c .* dv_c - dc_c   dg = dv_c - dW f - W df
+ *   dh = dr + dB'g + B' dg   dk = -G^-1 (dh + dG k)
+ *   dV_p += dA'Y + Y'dA + A' dW A + dH'K + K'dH + K' dG K   (exactly symmetric)
+ *   dv_p += dA'g + A' dg + dK'h + K' dh
+ * where every node starts from dV_i = sym(dQ_i), dv_i = dq_i.  Each convention is the
+ * transpose of one of sipoc_lqr_policy_vjp, so <cot, JVP(t)> = <t, VJP(cot)> for every tangent:
+ * dQ and dR enter through their symmetric parts (the full matrices are read), and the root's
+ * dc and ddelta are not read (K and V do not depend on them).  Tangents of q, r and c alone give
+ * dK = 0 and dV = 0 exactly.
+ *   in      : R, M, r, A, B, c, delta of the forward are read; Q and q are not and may be NULL.
+ *   V, v    : the forward's policy arrays, required.  Only the lower triangle of V is read.
+ *   status  : the forward's per-problem FactorStatus, required.
+ *   tangent : required; any of its nine arrays may be NULL, which is not read and gives
+ *             bitwise the same result as zeros.
+ *   dpolicy : required; any of its four arrays may be NULL, and is then not written.
+ * Every requested output array is written in full: zeros in problems whose status != 0 and in
+ * the padding lanes batch <= b < batch_stride.  dV is exactly symmetric.  Any structure
+ * sipoc_lqr_factor_solve_policy accepts.  FP64, engine layout, 16-byte aligned arrays.  Trees
+ * and shapes without a specialised kernel use an engine-owned workspace sized on the first
+ * call, so the call can be recorded in a graph once it has run eagerly. */
+sipoc_error sipoc_lqr_policy_jvp(sipoc_engine *engine, const sipoc_lqr_input *in,
+                                 const double *V, const double *v, const int *status,
+                                 const sipoc_lqr_input *tangent,
+                                 const sipoc_lqr_policy *dpolicy, void *stream);
+
 /* ---- layout conversion (device <-> device) ------------------------------ */
 /* src: problem-major [batch][size]; dst: engine layout [size][batch_stride]. */
 sipoc_error sipoc_pack(sipoc_engine *engine, const double *src, double *dst,

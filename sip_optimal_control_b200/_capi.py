@@ -202,6 +202,7 @@ def _load() -> ctypes.CDLL:
     lib.sipoc_lqr_factor_solve_policy.argtypes = [E, LI, LO, ctypes.POINTER(LqrPolicy), P, P]
     lib.sipoc_lqr_policy_vjp.argtypes = [E, LI, P, P, P, ctypes.POINTER(LqrPolicyCotangent),
                                          ctypes.POINTER(LqrGrad), P]
+    lib.sipoc_lqr_policy_jvp.argtypes = [E, LI, P, P, P, LI, ctypes.POINTER(LqrPolicy), P]
     lib.sipoc_status_stats.argtypes = [E, P, P, P]
     lib.sipoc_pack.argtypes = [E, P, P, ctypes.c_int64, P]
     lib.sipoc_unpack.argtypes = [E, P, P, ctypes.c_int64, P]

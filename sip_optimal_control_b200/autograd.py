@@ -19,6 +19,11 @@ Conventions (include/sipoc.h, sipoc_lqr_vjp):
 for the cotangents of x, u, y and ``sipoc_lqr_policy_vjp`` (the adjoint Riccati sweep) for
 those of K, k, V, v, each only when one of its cotangents is given, and sums the two.  It has
 no forward mode: ``forward_ad`` and ``torch.func.jvp`` through it raise torch's own error.
+``factor_solve_policy_fwd(lqr, inp)`` is the same function with forward mode as well: its
+tangent is ``sipoc_lqr_jvp`` for x, u, y plus ``sipoc_lqr_policy_jvp`` (the tangent Riccati
+sweep, leaves to root) for K, k, V, v.  torch asks for all outputs' tangents at once, so a
+forward-mode call always pays for both, even if only the policy's tangent is used; call
+``LQR.policy_jvp`` directly to pay for the policy sweep alone.
 
 ``kkt_factor_solve(cp, model, w, r1, r2, r3, b)`` does the same for the Newton-KKT solve
 (``CallbackProvider.factor`` + ``solve``) and returns ``(sol, ok)``; sol carries gradients
@@ -147,6 +152,36 @@ def factor_solve_policy(lqr, inp: dict):
     """Differentiable ``lqr.factor_solve_policy``: returns (x, u, y, K, k, V, v, status),
     status not differentiable.  ``inp`` as for ``factor_solve``.  Reverse mode only."""
     return _FactorSolvePolicy.apply(lqr, *(inp[k] for k in LQR_INPUT_FIELDS))
+
+
+class _FactorSolvePolicyFwd(_FactorSolvePolicy):
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        _FactorSolvePolicy.setup_context(ctx, inputs, output)
+        lqr, *arrays = inputs
+        x, u, y, _K, _k, V, v, status = output
+        ctx.save_for_forward(*arrays, x, u, y, V, v, status)
+
+    @staticmethod
+    def jvp(ctx, _lqr_t, *tangents):
+        n = len(LQR_INPUT_FIELDS)
+        with torch._C._DisableFuncTorch():
+            saved = [_plain(a) for a in ctx.saved_tensors]
+            inp = dict(zip(LQR_INPUT_FIELDS, saved[:n]))
+            x, u, y, V, v, status = saved[n:]
+            # forward_ad may hand out stride-0 expanded tangents; None is a zero tangent
+            tan = {k: _plain(t) for k, t in zip(LQR_INPUT_FIELDS, tangents) if t is not None}
+            res = ctx.lqr.jvp({k: inp[k] for k in _LQR_KEPT}, dict(x=x, u=u, y=y), tan)
+            pol = ctx.lqr.policy_jvp(inp, dict(V=V, v=v), status, tan)
+        return res["x"], res["u"], res["y"], pol["K"], pol["k"], pol["V"], pol["v"], None
+
+
+def factor_solve_policy_fwd(lqr, inp: dict):
+    """``factor_solve_policy`` with forward mode as well (``forward_ad``, ``torch.func.jvp``,
+    ``gradcheck(..., check_forward_ad=True)``): the same outputs and backward, and a tangent of
+    (x, u, y, K, k, V, v) from ``lqr.jvp`` and ``lqr.policy_jvp``.  Both tangent sweeps run on
+    every forward-mode call."""
+    return _FactorSolvePolicyFwd.apply(lqr, *(inp[k] for k in LQR_INPUT_FIELDS))
 
 
 _KKT_VECTORS = ("w", "r1", "r2", "r3", "b")

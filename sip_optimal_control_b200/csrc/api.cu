@@ -19,6 +19,7 @@
 #include "kkt_vjp.cuh"
 #include "lqr_vjp.cuh"
 #include "policy.cuh"
+#include "policy_jvp.cuh"
 #include "policy_vjp.cuh"
 #include "scan.cuh"
 #include "model_scatter.cuh"
@@ -111,6 +112,7 @@ struct sipoc_engine {
   int *vjp_status = nullptr;   // status / ok of sipoc_*_vjp / _jvp when the caller passes none (lazy)
   double *policy_V = nullptr;  // V rebuilt in a padded plan's shape, before extraction (lazy)
   double *policy_vjp_ws = nullptr;  // edge scratch and per-node Vb, vb of the generic policy VJP (lazy)
+  double *policy_jvp_ws = nullptr;  // edge scratch and per-node dV, dv of the generic policy JVP (lazy)
 
   // Parallel-in-time factor + solve (scan.cu): long uniform chains, small batches.
   struct Scan {
@@ -1485,6 +1487,47 @@ sipoc_error sipoc_lqr_policy_vjp(sipoc_engine *e, const sipoc_lqr_input *in, con
   }
   e->launches += 1;
   return check_launch(e, "lqr policy vjp");
+}
+
+// Forward mode of the policy (policy_jvp.cuh): the tangent Riccati sweep, leaves to root.
+// Uniform chains at the shapes of the thread and four-lane plans run the sub-warp kernel,
+// every other structure the generic one; the choice depends on the structure only.
+sipoc_error sipoc_lqr_policy_jvp(sipoc_engine *e, const sipoc_lqr_input *in, const double *V,
+                                 const double *v, const int *status,
+                                 const sipoc_lqr_input *tangent, const sipoc_lqr_policy *dpolicy,
+                                 void *stream) {
+  if (e == nullptr) return SIPOC_INVALID_ARGUMENT;
+  if (in == nullptr || !in->M || !in->R || !in->r || !in->A || !in->B || !in->c || !in->delta ||
+      V == nullptr || v == nullptr || status == nullptr || tangent == nullptr ||
+      dpolicy == nullptr)
+    return fail(e, SIPOC_INVALID_ARGUMENT,
+                "NULL LQR input / policy V, v / status / tangent / dpolicy");
+  const LqrPolicy out{dpolicy->K, dpolicy->k, dpolicy->V, dpolicy->v};
+  if (!out.K && !out.k && !out.V && !out.v) return SIPOC_OK;
+  DeviceGuard guard(e->device);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const HostStructure &h = e->hs;
+  const PolicyVjpIn pin{to_in(in), V, v};
+  const LqrIn tan = to_in(tangent);
+  if (h.is_chain && h.is_uniform && h.E >= 1 && policy_jvp_subwarp_shape(h.n[0], h.m[0])) {
+    bool ok;
+    {
+      ProfScope ps(&e->prof, "policy_jvp_subwarp", s);
+      ok = launch_policy_jvp_subwarp(h.n[0], h.m[0], h.E, pin, tan, out, status, e->batch, e->ld,
+                                     s);
+    }
+    if (!ok) return fail(e, SIPOC_CUDA_ERROR, "policy JVP: sub-warp kernel not configured");
+  } else {
+    if (e->policy_jvp_ws == nullptr) {
+      const sipoc_error rc = alloc_doubles(e, &e->policy_jvp_ws, policy_jvp_generic_ws_elems(h));
+      if (rc != SIPOC_OK) return rc;
+    }
+    ProfScope ps(&e->prof, "policy_jvp_generic_kernel", s);
+    launch_policy_jvp_generic(e->dt, h, pin, tan, out, e->policy_jvp_ws, status, e->batch, e->ld,
+                              s);
+  }
+  e->launches += 1;
+  return check_launch(e, "lqr policy jvp");
 }
 
 sipoc_error sipoc_status_stats(sipoc_engine *e, const int *status, double *stats,

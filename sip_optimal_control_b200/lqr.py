@@ -397,8 +397,9 @@ class LQR:
         ``u_e = K_e x_parent(e) + k_e`` (K: m_e x n_parent column-major, the element count of
         M; k: that of r), per node ``y_i = V_i x_i + v_i`` (V: n_i x n_i, that of Q; v: that
         of q) -- and ``status``.  ``policy`` may supply the output tensors.  Failed problems
-        and padding lanes get zeros.  The outputs are plain tensors; the differentiable variant
-        is ``autograd.factor_solve_policy``, whose backward runs ``policy_vjp``."""
+        and padding lanes get zeros.  The outputs are plain tensors; the differentiable variants
+        are ``autograd.factor_solve_policy``, whose backward runs ``policy_vjp``, and
+        ``autograd.factor_solve_policy_fwd``, which adds forward mode through ``policy_jvp``."""
         if self.traversal_status_ != FactorStatus.SUCCESS:
             return dict(status=self._invalid())
         e = self.engine
@@ -488,6 +489,40 @@ class LQR:
                                           ctypes.byref(sc), ctypes.byref(sg),
                                           e.stream_ptr(stream)))
         return grads
+
+    def policy_jvp(self, inp: dict, policy: dict, status, tan: dict, want=None, dpolicy=None,
+                   stream=None) -> dict:
+        """Forward-mode derivative of the policy of ``factor_solve_policy``
+        (sipoc_lqr_policy_jvp; include/sipoc.h).
+
+        ``inp`` holds the forward's inputs (Q and q are not read), ``policy`` its ``V`` and
+        ``v`` (both required: the tangent sweep recomputes W, G, K and k from them), ``status``
+        its per-problem FactorStatus.  ``tan`` holds the tangents of any subset of the nine
+        input names (engine layout); an absent name is a zero tangent and is not read.
+        ``want`` is a subset of ``{"K", "k", "V", "v"}`` (default: all four); the others are
+        not written.  ``dpolicy`` may supply the output tensors.  Returns a dict with the
+        tangent dK, dk, dV, dv of each wanted name, keyed K, k, V, v.  dQ and dR enter through
+        their symmetric parts; failed problems and padding lanes get zeros."""
+        e = self.engine
+        want = set(_capi.LQR_POLICY_FIELDS if want is None else want)
+        unknown = want - set(_capi.LQR_POLICY_FIELDS)
+        if unknown:
+            raise ValueError(f"not a policy array: {sorted(unknown)}")
+        unknown = set(tan) - set(_capi.LQR_INPUT_FIELDS)
+        if unknown:
+            raise ValueError(f"not an LQR input: {sorted(unknown)}")
+        given = {} if dpolicy is None else dpolicy
+        arrays = {k: given[k] if k in given else e.empty(e.lqr_sizes[_capi.LQR_POLICY_SIZE_OF[k]])
+                  for k in _capi.LQR_POLICY_FIELDS if k in want}
+        si, st = _lqr_input_struct(inp), _lqr_input_struct(tan)
+        sp = _capi.LqrPolicy()
+        for k in _capi.LQR_POLICY_FIELDS:
+            setattr(sp, k, arrays[k].data_ptr() if k in arrays else None)
+        e._check(lib.sipoc_lqr_policy_jvp(e._handle, ctypes.byref(si), policy["V"].data_ptr(),
+                                          policy["v"].data_ptr(), status.data_ptr(),
+                                          ctypes.byref(st), ctypes.byref(sp),
+                                          e.stream_ptr(stream)))
+        return arrays
 
     def jvp(self, inp: dict, out: dict, tan: dict, dsol=None, rhs=None, status=None,
             stream=None) -> dict:
